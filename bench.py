@@ -1,14 +1,14 @@
 #!/usr/bin/env python
 """Headline benchmark: fused SQ implicit-loss forward+backward throughput (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: ``ImplicitLoss(64, dev, 1.5, 260)(images, pred)`` followed by
 ``.backward()`` on BASELINE config 2 (batch 256, 64^3 grid, fp32) -- 67 108 864 points per GPU.  Under torchrun
 (N > 1) every rank runs its own batch (the path shards by sample, no data-path collective: weak scaling) and the
 step time is the max over ranks.
 
-Printed line (rank 0), see the driver contract:
+Printed line (rank 0):
   ``value``        Gpoints/s with inputs resident in HBM (CUDA events over exactly K graph-replayed steps)
   ``dense``        the same call on a second workload, sizes a ~ U(0.5, 1): objects fill the grid, culling cannot help
   ``e2e``          host buffers in, host results out, copies inside the timed region: 8-bit depth maps and fp32 parameters in
@@ -18,6 +18,14 @@ Printed line (rank 0), see the driver contract:
                    build of the same sources, ``walked_fraction``, ``evaluated_gpoints_per_s``; DRAM traffic from the ncu capture
   ``cpu_baseline`` the UNMODIFIED reference (staged under oracle/_ref) on the box's host cores on a bounded sample
 ``--impl reference`` times that CPU path alone (same ``config``; ``--steps`` / ``--warmup`` honoured).
+
+``--steps K`` sets the timed window of ``value`` and of ``one_batch_at_a_time`` exactly.  The secondary windows time their
+own counts, each reported next to its figure: ``dense`` max(4, min(K, 80)) steps, ``e2e`` max(4, K), its blocking fp32 call
+and the kernel-alone times at most 20.
+
+``--dump-outputs DIR`` writes what the last timed step returned to its caller -- the loss (float64) and the gradient with
+respect to the parameters (float32, B x 12) of the headline workload and of ``dense`` -- as DIR/<name>.npy (``_rank<r>``
+appended under torchrun).  The inputs are seeded, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -104,7 +112,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, max(0, args.warmup)
     cb, mean = cpu_reference(steps, warmup)
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": steps, "warmup": warmup, "ms_per_step": mean * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -399,6 +407,8 @@ def run_gpu(args):
     ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if rank == 0 else None
     assert torch.isfinite(loss).item() and torch.isfinite(grad).all().item()
+    # copied now: later replays of the same graphs overwrite their output buffers
+    outputs = {"loss": loss.detach().cpu(), "grad": grad.cpu()}
     # the same K steps one batch at a time (no overlap between consecutive steps)
     main.run(8, sequential=True)
     barrier()
@@ -412,10 +422,11 @@ def run_gpu(args):
     dense.run(8)
     barrier()
     ev0.record()
-    dense.run(dsteps)
+    dense_loss, dense_grad = dense.run(dsteps)
     ev1.record()
     barrier()
     dms = ev0.elapsed_time(ev1)
+    outputs.update(dense_loss=dense_loss.detach().cpu(), dense_grad=dense_grad.cpu())
     kms = main.kernel_ms(_lib.lib(), min(steps, 20))
     dkms = dense.kernel_ms(_lib.lib(), min(steps, 12))
     eager_ms = None
@@ -573,6 +584,11 @@ def run_gpu(args):
         if world == 1:
             line["cpu_baseline"] = cpu_reference(5, 1)[0]
         print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        suffix = f"_rank{rank}" if world > 1 else ""
+        for name, t in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + suffix + ".npy"), t.numpy())
     if world > 1:
         dist.destroy_process_group()
 
@@ -584,7 +600,12 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--eager", action="store_true", help="time eager launches instead of CUDA-graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's loss and gradient as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path only")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,5 +1,6 @@
 """ctypes loader for the host build of sq_core.cuh (tests/emu/emu.cpp) -- TEST TOOL ONLY."""
 import ctypes
+import hashlib
 import os
 import subprocess
 import tempfile
@@ -15,13 +16,22 @@ def lib():
     global _lib
     if _lib is None:
         flags = os.environ.get("SQ_EMU_FLAGS", "").split()            # experiments: -DSQ_KREFINE=32.0f ...
-        tag = ("_" + "".join(c if c.isalnum() else "_" for c in "".join(flags))) if flags else ""
-        out = os.path.join(tempfile.gettempdir(), f"libsqemu_{os.getuid()}{tag}.so")
         src = os.path.join(HERE, "emu.cpp")
-        hdr = os.path.join(ROOT, "sq_recovery_b200", "csrc", "sq_core.cuh")
-        if not os.path.exists(out) or os.path.getmtime(out) < max(os.path.getmtime(src), os.path.getmtime(hdr)):
-            subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", *flags, "-I", os.path.dirname(hdr),
-                                   "-x", "c++", src, "-o", out])
+        csrc = os.path.join(ROOT, "sq_recovery_b200", "csrc")
+        # the temporary directory is shared with other checkouts: the cached build is named after what it was built from
+        h = hashlib.sha256(" ".join(flags).encode())
+        for path in (src, os.path.join(csrc, "sq_core.cuh"), os.path.join(csrc, "sq_tables.inc")):
+            h.update(open(path, "rb").read())
+        out = os.path.join(tempfile.gettempdir(), f"libsqemu_{os.getuid()}_{h.hexdigest()[:16]}.so")
+        if not os.path.exists(out):
+            tmp = f"{out}.{os.getpid()}"
+            try:
+                subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", *flags, "-I", csrc,
+                                       "-x", "c++", src, "-o", tmp])
+                os.replace(tmp, out)
+            finally:
+                if os.path.exists(tmp):
+                    os.remove(tmp)
         _lib = ctypes.CDLL(out)
     return _lib
 

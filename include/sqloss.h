@@ -78,6 +78,18 @@ int sq_implicit_loss_heads(const void* raw_heads, int dtype, int batch, int n, d
                            double* loss_out, double* per_sample, void* grad_raw, float* depth_out,
                            void* scratch, size_t scratch_bytes, sq_stream_t stream);
 
+/* Vector-Jacobian product of ImplicitLoss.depth_projection (torch/classes.py:232-282):
+ *   grad_depth  [batch,n,n] fp32, contiguous, image orientation (the layout of depth_out)
+ *   grad_pred   [batch,12] (pred_dtype) = sum_pix grad_depth[b,pix] * d depth[b,pix] / d pred[b]
+ *               (clamp masks as in the loss; quaternion not normalised)
+ * Same scratch contract as the other entry points; asynchronous on `stream`.  Self-contained: it reads nothing an earlier
+ * call left in the scratch buffer (it renders the columns again), so any calls may run between the forward and this one.
+ * For the MAE objective the fused sq_implicit_loss is cheaper: it needs one walk of the grid, this path two.
+ */
+int sq_depth_projection_vjp(const void* pred, int pred_dtype, int batch, int n, double step, double z0,
+                            float tau, float sharpness, const float* grad_depth, void* grad_pred,
+                            void* scratch, size_t scratch_bytes, sq_stream_t stream);
+
 /* ExplicitLoss.__call__ (torch/classes.py:138-201): mean_b( mult * mean_pts (o_true - o_pred)^2 ),
  * o = sigmoid(sharpness (1 - F)); the reference uses sharpness 5, mult 100 (:187, :198).
  *   grad_pred   [batch,12] d loss / d pred (params_dtype)              (NULL = forward only)

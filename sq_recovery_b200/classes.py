@@ -32,7 +32,7 @@ def _preprocess_sq(p: torch.Tensor) -> torch.Tensor:
     return torch.cat([a.clamp(0.05, 1), e.clamp(0.1, 1), t.clamp(0, 1), q], dim=-1)
 
 
-def _no_history(p: torch.Tensor, what: str) -> None:
+def _no_history(p: torch.Tensor, what: str, instead: str = "") -> None:
     """The grid-returning conveniences are forward-only here (the reference returns fp64 grids WITH autograd history,
     torch/classes.py:138-189, 232-282, 394-426).  Differentiating through them would silently yield no gradient, so a
     tensor that asks for one is refused instead."""
@@ -40,7 +40,7 @@ def _no_history(p: torch.Tensor, what: str) -> None:
         raise RuntimeError(
             f"sq_recovery_b200: {what}() is forward-only (fp32 grid, no autograd history); it was given a tensor that "
             "requires grad.  Call it under torch.no_grad() / on p.detach(), or differentiate through the loss call "
-            "(loss(true, pred).backward()), which is fused.")
+            f"(loss(true, pred).backward()), which is fused.{instead}")
 
 
 class _GridLoss:
@@ -103,8 +103,20 @@ class ImplicitLoss(_GridLoss):
 
     def depth_projection(self, p):
         """(B, R, R) depth render in image orientation (classes.py:232-282), fp32, no autograd."""
-        _no_history(p, "depth_projection")
+        _no_history(p, "depth_projection", "  For a depth render to differentiate through (any image-space loss), "
+                    "use render(p).")
         return Fn.depth_projection(p, self._n, self._step, self._z0, float(self.tau), float(self.sigmoid_sharpness))
+
+    def render(self, p):
+        """(B, R, R) fp32 depth render in image orientation, differentiable w.r.t. ``p`` (the reference's depth_projection
+        with autograd history, classes.py:232-282): the same bits as ``depth_projection``; its backward is one CUDA
+        vector-Jacobian product, so any image-space loss (L2, Huber, masks, weights, sums of terms) can be trained through
+        it.  For the plain MAE against a target image, ``self(true, pred)`` is cheaper: it is fused into one walk.
+        Under torch.no_grad(), or for a ``p`` that does not require grad, a plain tensor."""
+        args = (self._n, self._step, self._z0, float(self.tau), float(self.sigmoid_sharpness))
+        if torch.is_grad_enabled() and isinstance(p, torch.Tensor) and p.requires_grad:
+            return Fn.DepthProjectionFn.apply(p, *args)
+        return Fn.depth_projection(p, *args)
 
     def __call__(self, true, pred):
         return Fn.ImplicitLossFn.apply(true, pred, self._n, self._step, self._z0, float(self.tau),

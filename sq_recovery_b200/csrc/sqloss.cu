@@ -740,7 +740,9 @@ __device__ unsigned long long g_phase[8];
 constexpr size_t kImplicitBwdSmemPerWarp = (size_t)kBwdPool * 4 * sizeof(float) + 11 * 32 * sizeof(float);
 static_assert(kImplicitBwdSmemPerWarp % 32 == 0, "per-warp regions stay 32-byte aligned (BwdQueue::where carries the lane in its low bits)");
 
-template <bool BWD, int THREADS, int MINB, int CPTMAX>      // CPTMAX: upper limit of L.cpt
+// VJP (with BWD; sq_depth_projection_vjp): `target` is the upstream gradient dL/d depth [batch, n, n] in image orientation and
+// takes the place of sign(depth - target) as the column's weight; no loss, no depth, partial-row slots 17-19 stay 0.
+template <bool BWD, int THREADS, int MINB, int CPTMAX, bool VJP = false>      // CPTMAX: upper limit of L.cpt
 __global__ void __launch_bounds__(THREADS, MINB)
 implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, ImplicitParams P, int total_items,
                 Control* __restrict__ ctl, const int* __restrict__ queue, int cap,
@@ -768,6 +770,7 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
 #else
     float* const tile_w = tiles_static[threadIdx.x >> 5];
 #endif
+    static_assert(!VJP || BWD, "the VJP mode is a mode of the fwd+bwd kernel");
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     Sample& S = Ssh[warp];
 #if defined(SQ_BWD_COMPACT) && !defined(SQ_TABLES_GLOBAL)
@@ -832,7 +835,7 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
             bool folded = false;
             ColIter it;
             it.init(L, chunk, lane);
-            // the item's target pixels: loads issued up front (they miss to HBM), used after the z walks
+            // the item's target pixels (VJP: upstream pixels): loads issued up front (they miss to HBM), used after the z walks
             float tvs[CPTMAX];
             {
                 ColIter pt = it;
@@ -840,7 +843,9 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
                 for (int k = 0; k < CPTMAX; ++k) {
                     tvs[k] = 0.f;
                     if (target && k < L.cpt) {
-                        if (pt.valid(L)) tvs[k] = __ldg(target + (size_t)b * tstride + row_off[g.n - 1 - pt.ib] + col_off[pt.ia]);
+                        if (pt.valid(L))
+                            tvs[k] = VJP ? __ldg(target + ((size_t)b * g.n + (g.n - 1 - pt.ib)) * g.n + pt.ia)
+                                         : __ldg(target + (size_t)b * tstride + row_off[g.n - 1 - pt.ib] + col_off[pt.ia]);
                         pt.next(L);
                     }
                 }
@@ -926,7 +931,7 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
 #endif
 #if defined(SQ_BWD_COMPACT)
                 if (BWD) {
-                    // sign of (depth - target) per column; 0 for masked lanes
+                    // sign of (depth - target) per column (VJP: the upstream pixel); 0 for masked lanes
                     float wsg = 0.f;
                     // the target pixel (issued before the walk, a miss to HBM) is first touched HERE: without the fence the
                     // compiler forms |tv| right behind the load and the warp waits out the miss before it starts walking
@@ -934,7 +939,9 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
 #pragma unroll
                     for (int q = 1; q < CPTMAX; ++q) tv = k == q ? tvs[q] : tv;
                     asm volatile("" : "+f"(tv));
-                    if (valid) {
+                    if (valid && VJP) {
+                        wsg = tv;
+                    } else if (valid) {
                         if (depth_out) depth_out[((size_t)b * g.n + row) * g.n + col] = depth;
                         const float diff = depth - tv;
                         loss_sum += fabsf(diff) - fabsf(tv);
@@ -983,7 +990,7 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
                             const float tau = P.tl * (float)kLn2;
 #ifdef SQ_DEPTH_SHIFT       // the refined occupancies' first-order effect on the rendered depth: measured below the loss's other
                             // fp32 errors on every workload (profiles/tune_r02.txt) and 2 us per call -> off
-                            if (head != kNoLink) loss_sum = fmaf(wsg * tau * g.inv_n, queue_depth_shift(qwarp, head, U), loss_sum);
+                            if (!VJP && head != kNoLink) loss_sum = fmaf(wsg * tau * g.inv_n, queue_depth_shift(qwarp, head, U), loss_sum);
 #endif
 #ifndef SQ_EARLY_CLAIM
                             if (staged && wp.claim_finish()) pre.fetch(samples + L.sample_of(wp.next), lane);
@@ -1031,19 +1038,19 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
                 } else
 #endif
                 if (valid) {
-                    if (depth_out) depth_out[((size_t)b * g.n + row) * g.n + col] = depth;
+                    if (depth_out && !VJP) depth_out[((size_t)b * g.n + row) * g.n + col] = depth;
                     if (target) {
                         float tv = tvs[0];
 #pragma unroll
                         for (int q = 1; q < CPTMAX; ++q) tv = k == q ? tvs[q] : tv;
                         asm volatile("" : "+f"(tv));           // first touch of the pixel after the walk (see above)
-                        const float diff = depth - tv;
-                        loss_sum += fabsf(diff) - fabsf(tv);
+                        const float diff = VJP ? tv : depth - tv;
+                        if (!VJP) loss_sum += fabsf(diff) - fabsf(tv);
                         if (BWD && diff != 0.f) {
                             float v[kRedStride];
                             Acc acc;
                             if (folded) { tile_get(tile_w, v); array_to_acc(v, acc); } else acc_zero(acc);
-                            implicit_fold(acc, cg, diff > 0.f ? 1.f : -1.f, dxy[0], dxy[1]);
+                            implicit_fold(acc, cg, VJP ? diff : (diff > 0.f ? 1.f : -1.f), dxy[0], dxy[1]);
                             acc_to_array(acc, v);
                             v[18] = v[19] = 0.f;
                             tile_put(tile_w, v);
@@ -1509,6 +1516,22 @@ int persistent_blocks(int items, int warps_per_block, int min_blocks_per_sm) {
     return need < fill ? need : fill;
 }
 
+// Static + dynamic shared memory of the fwd+bwd kernels exceed 48 KB: opt in once per kernel and device (not a stream
+// operation).  The kernel is a template argument so that every kernel has its own `opted` table (the fwd+bwd kernels
+// share one function-pointer type).
+template <auto KERNEL>
+cudaError_t opt_in_dyn_smem(size_t dyn) {
+    static bool opted[64] = {false};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev >= 0 && dev < 64 && !opted[dev]) {
+        const cudaError_t e = cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+        if (e != cudaSuccess) return e;
+        opted[dev] = true;
+    }
+    return cudaSuccess;
+}
+
 int launch_prep(const void* params, int dtype, int batch, bool clamp, const Grid& g, SampleFull* out, Control* ctl,
                 cudaStream_t st) {
     if (dtype != SQ_F32 && dtype != SQ_F64) return (int)cudaErrorInvalidValue;
@@ -1644,16 +1667,7 @@ static int implicit_loss_impl(const void* pred, int pred_dtype, int batch, int n
         if (grad_pred) {
             const int blocks = persistent_blocks(items, SQ_IMPB_THREADS / 32, SQ_IMPB_MINB);
             constexpr size_t dyn = kImplicitBwdSmemPerWarp * (SQ_IMPB_THREADS / 32);
-            {   // static + dynamic shared memory exceed 48 KB: opt in once per device (not a stream operation)
-                static bool opted[64] = {false};
-                int dev = 0;
-                cudaGetDevice(&dev);
-                if (dev >= 0 && dev < 64 && !opted[dev]) {
-                    SQ_TRY(cudaFuncSetAttribute(implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT>,
-                                                cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-                    opted[dev] = true;
-                }
-            }
+            SQ_TRY((opt_in_dyn_smem<implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT>>(dyn)));
             SQ_TRY(launch_dependent(implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT>, blocks, SQ_IMPB_THREADS, dyn, st, pdl,
                                     s.pred, g, L, P, items, s.ctl, queue, s.queue_cap, target, target_stride_b, row_off, col_off,
                                     s.partials, depth_out));
@@ -1693,6 +1707,51 @@ int sq_implicit_loss_heads(const void* raw_heads, int dtype, int batch, int n, d
                            float* depth_out, void* scratch, size_t scratch_bytes, sq_stream_t stream) {
     return implicit_loss_impl(raw_heads, dtype, batch, n, step, z0, target, target_stride_b, row_off, col_off, tau, sharpness,
                               loss_out, per_sample, grad_raw, depth_out, scratch, scratch_bytes, stream, true);
+}
+
+// The fwd+bwd pipeline with the upstream pixel as the column weight (implicit_kernel VJP mode): plan (no pixel sum; the
+// item classes still let finalize skip proven-empty items, whose columns carry no weight above the cut for any upstream),
+// column kernel, finalize with the scale of d depth / d theta alone.  Nothing is read that an earlier call left behind.
+int sq_depth_projection_vjp(const void* pred, int pred_dtype, int batch, int n, double step, double z0,
+                            float tau, float sharpness, const float* grad_depth, void* grad_pred,
+                            void* scratch, size_t scratch_bytes, sq_stream_t stream) {
+    Scratch s;
+    int rc = check_scratch(batch, n, scratch, scratch_bytes, &s);
+    if (rc) return rc;
+    if (!grad_depth || !grad_pred) return (int)cudaErrorInvalidValue;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const Grid g = make_grid(n, step, z0);
+    const Layout L = make_layout(n, SQ_IMPB_CPT);
+    // the weight cut of one sample (batch 1): a VJP's gradient of sample b does not depend on the batch
+    const ImplicitParams P{sharpness * kLog2e, tau * kLog2e, implicit_cull_bound(sharpness * kLog2e), implicit_active_bits(sharpness * kLog2e, n, 1)};
+    rc = launch_plan(pred, nullptr, pred_dtype, batch, true, g, L, P.bound, s, nullptr, s.item_class, nullptr, st, false,
+                     SQ_WALK_ESTIMATE ? 32.0f / P.tl : 0.f);
+    if (rc) return rc;
+    const int items = batch * L.rows_per_sample;
+    const int* queue = L.rows_per_sample <= kPlanMaxItems ? s.queue : nullptr;
+#ifdef SQ_PDL
+    const bool pdl = (t_ev_before == nullptr && t_ev_after == nullptr);
+#else
+    const bool pdl = false;
+#endif
+    {
+        ColumnKernelTimer timer(st);
+        const int blocks = persistent_blocks(items, SQ_IMPB_THREADS / 32, SQ_IMPB_MINB);
+        constexpr size_t dyn = kImplicitBwdSmemPerWarp * (SQ_IMPB_THREADS / 32);
+        SQ_TRY((opt_in_dyn_smem<implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT, true>>(dyn)));
+        SQ_TRY(launch_dependent(implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT, true>, blocks, SQ_IMPB_THREADS, dyn,
+                                st, pdl, s.pred, g, L, P, items, s.ctl, queue, s.queue_cap, grad_depth, 0LL,
+                                static_cast<const int*>(nullptr), static_cast<const int*>(nullptr), s.partials,
+                                static_cast<float*>(nullptr)));
+    }
+    SQ_TRY(cudaGetLastError());
+    // d depth / d o_c = (tau / n) S_c and d o / d F = -k o (1 - o): the column sums carry o (1 - o) S_c x upstream
+    SQ_TRY(launch_dependent(finalize_kernel<FIN_IMPLICIT>, batch, kFinThreads, 0, st, pdl,
+                            s.pred, g, batch, L.rows_per_sample, s.partials, 0.0, -(double)sharpness * (double)tau / (double)n,
+                            pred_dtype, grad_pred, s.per_sample, static_cast<double*>(nullptr), static_cast<double*>(nullptr),
+                            &s.ctl->ticket, static_cast<const double*>(nullptr), queue ? s.item_class : nullptr));
+    SQ_TRY(cudaGetLastError());
+    return 0;
 }
 
 int sq_explicit_loss(const void* true_params, const void* pred, int params_dtype, int batch, int n, double step,

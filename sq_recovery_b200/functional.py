@@ -323,8 +323,12 @@ def iou_counts(true: torch.Tensor, pred: torch.Tensor, n: int, step: float, z0: 
 def depth_projection(pred: torch.Tensor, n: int, step: float, z0: float, tau: float, sharpness: float) -> torch.Tensor:
     """ImplicitLoss.depth_projection (torch/classes.py:232-282): (B, n, n) fp32 render, image orientation."""
     _require_cuda(pred, "pred")
-    dev = pred.device
     p, tag = _params(pred)
+    return _render(p, tag, n, step, z0, tau, sharpness)
+
+
+def _render(p: torch.Tensor, tag: int, n: int, step: float, z0: float, tau: float, sharpness: float) -> torch.Tensor:
+    dev = p.device
     B = p.shape[0]
     out = torch.empty((B, n, n), dtype=torch.float32, device=dev)
     scratch = _get_scratch(dev, B, n)
@@ -333,6 +337,36 @@ def depth_projection(pred: torch.Tensor, n: int, step: float, z0: float, tau: fl
                                          None, _ptr(out), _ptr(scratch), scratch.numel(), _stream(dev))
     _lib.check(rc, "sq_implicit_loss(depth)")
     return out
+
+
+class DepthProjectionFn(torch.autograd.Function):
+    """Differentiable ImplicitLoss.depth_projection: the forward is the forward-only render (same bits as
+    ``depth_projection``); the backward is the vector-Jacobian product kernel (sq_depth_projection_vjp), which walks the
+    grid again with the upstream pixels as column weights.  Any image-space loss on the render can be trained through it;
+    for the MAE against a target image the fused ImplicitLossFn is cheaper (one walk instead of two)."""
+
+    @staticmethod
+    def forward(ctx, pred, n, step, z0, tau, sharpness):
+        _require_cuda(pred, "pred")
+        p, tag = _params(pred)
+        ctx.p, ctx.tag, ctx.pred_dtype = p, tag, pred.dtype
+        ctx.args = (n, step, z0, tau, sharpness)
+        return _render(p, tag, n, step, z0, tau, sharpness)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, go):
+        p, (n, step, z0, tau, sharpness) = ctx.p, ctx.args
+        dev = p.device
+        B = p.shape[0]
+        g = go.float().contiguous()
+        grad = torch.empty_like(p)
+        scratch = _get_scratch(dev, B, n)
+        with _on_device(dev):
+            rc = _lib.lib().sq_depth_projection_vjp(_ptr(p), ctx.tag, B, n, step, z0, tau, sharpness, _ptr(g), _ptr(grad),
+                                                    _ptr(scratch), scratch.numel(), _stream(dev))
+        _lib.check(rc, "sq_depth_projection_vjp")
+        return grad.to(ctx.pred_dtype), None, None, None, None, None
 
 
 def field(params: torch.Tensor, n: int, step: float, z0: float, mode: int, sharpness: float = 0.0) -> torch.Tensor:

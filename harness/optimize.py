@@ -2,13 +2,15 @@
 """Batched superquadric refinement by gradient descent -- the loop of torch/visu.py:120-186 without the GUI, run for
 thousands of SQs at once (SURVEY 8f-4).
 
-    python harness/optimize.py [--pairs 4096] [--steps 200] [--render 32] [--loss explicit|implicit]
+    python harness/optimize.py [--pairs 4096] [--steps 200] [--render 32] [--loss explicit|implicit|voxels]
     python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 harness/optimize.py
 
 Per step and per SQ, exactly the reference's update (visu.py:176-186): params[:8] -= lr * grad[:8];
 q -= lr * grad[8:]; q <- q / |q|, with lr = 0.001 and the loss ExplicitLoss(render_size=32) (visu.py:71).  The reference
 optimises ONE pair (batch 1); here every pair must see the gradient of ITS OWN loss, so the batch-mean loss the classes
 return is scaled back by the batch size.  Pairs are sharded over the ranks; no collective during the descent.
+--loss voxels fits to voxel data instead of ground-truth parameters: the target is the binarised occupancy
+(occupancy(true) > 0.5) on ExplicitLoss(R)'s grid, the criterion 100 mean((soft_occupancy(pred) - voxels)^2) (VoxelLoss).
 Prints one JSON line on rank 0: steps/s, loss evaluations (grid points) per second, IoU(128) before / after.
 """
 import argparse
@@ -44,12 +46,30 @@ def descend(crit, true, pred, steps, lr=LR, record=None):
     return loss
 
 
+class VoxelLoss:
+    """100 mean((occupancy(pred) - voxels)^2) over the batch and the grid, with the call signature of the loss classes:
+    crit(voxels, pred).  `occupancy` maps (B, 12) parameters to a differentiable (B, n, n, n) occupancy grid --
+    ExplicitLoss.soft_occupancy, or the oracle's ExplicitLoss.occupancy; `voxels` is the target grid on the same points."""
+
+    def __init__(self, occupancy):
+        self.occupancy = occupancy
+
+    def __call__(self, voxels, pred):
+        return 100.0 * ((self.occupancy(pred) - voxels) ** 2).mean()
+
+
+def voxelize(explicit_loss, params):
+    """Binarised occupancy (occupancy > 0.5, i.e. F < 1) of `params` on `explicit_loss`'s grid, fp32 (B, n, n, n)."""
+    with torch.no_grad():
+        return (explicit_loss.occupancy(params) > 0.5).float()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--pairs", type=int, default=4096)
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--render", type=int, default=32)
-    ap.add_argument("--loss", default="explicit", choices=["explicit", "implicit"])
+    ap.add_argument("--loss", default="explicit", choices=["explicit", "implicit", "voxels"])
     args = ap.parse_args()
     import sq_recovery_b200 as S
     from sq_recovery_b200 import distributed as D
@@ -66,6 +86,9 @@ def main():
     R = args.render
     if args.loss == "explicit":
         crit, target, pts = S.ExplicitLoss(R, dev), true, (b1 - b0) * (R + 1) ** 3
+    elif args.loss == "voxels":
+        grid = S.ExplicitLoss(R, dev)
+        crit, target, pts = VoxelLoss(grid.soft_occupancy), voxelize(grid, true), (b1 - b0) * grid._n ** 3
     else:
         crit = S.ImplicitLoss(R, dev, 1.5, 260)
         target = S.ImplicitLoss(256, dev, 1.5, 260).depth_projection(true).unsqueeze(1).contiguous()

@@ -138,6 +138,19 @@ int sq_least_squares_points(const void* pred, int pred_dtype, int batch, const f
 int sq_field(const void* params, int params_dtype, int batch, int n, double step, double z0,
              int mode, float sharpness, float* out, void* scratch, size_t scratch_bytes, sq_stream_t stream);
 
+/* Vector-Jacobian product of ExplicitLoss.occupancy / sq_field mode 1 (torch/classes.py:138-189):
+ *   grad_field  [batch,n,n,n] fp32, contiguous, index order [x][y][z] (the layout sq_field writes)
+ *   grad_params [batch,12] (params_dtype) = sum_vox grad_field[b,vox] * d occ[b,vox] / d params[b]
+ *               (clamp masks and zero fix-up as in the loss; quaternion not normalised)
+ * Same scratch contract as the other entry points; asynchronous on `stream`.  Self-contained: it reads nothing an earlier
+ * call left in the scratch buffer, so any calls may run between the forward and this one.  Voxels whose weight
+ * o (1 - o) is below 2^-36 are dropped (DESIGN.md 2).  For the MSE against the occupancy of known parameters the fused
+ * sq_explicit_loss is cheaper: it needs neither the field nor its gradient in memory.
+ */
+int sq_occupancy_vjp(const void* params, int params_dtype, int batch, int n, double step, double z0,
+                     float sharpness, const float* grad_field, void* grad_params,
+                     void* scratch, size_t scratch_bytes, sq_stream_t stream);
+
 /* ---- host-buffer entry points (what a non-torch caller binds; H2D/D2H copies happen inside) -------------------
  * An sq_ctx owns a stream, device buffers and pinned staging buffers on one device; buffers grow on demand and are
  * reused across calls.  The *_host calls return after the results are in the caller's host memory.

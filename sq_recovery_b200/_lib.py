@@ -26,6 +26,8 @@ _PROTOS = {
                                        c_size_t, c_void_p]),
     "sq_depth_projection_vjp": (c_int, [c_void_p, c_int, c_int, c_int, c_double, c_double, c_float, c_float, c_void_p,
                                         c_void_p, c_void_p, c_size_t, c_void_p]),
+    "sq_occupancy_vjp": (c_int, [c_void_p, c_int, c_int, c_int, c_double, c_double, c_float, c_void_p, c_void_p, c_void_p,
+                                 c_size_t, c_void_p]),
     "sq_explicit_loss": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_double, c_float, c_float,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "sq_iou_counts": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_double, c_void_p, c_void_p,

@@ -85,7 +85,20 @@ class ExplicitLoss(_GridLoss):
 
     def occupancy(self, p):
         """(B, n, n, n) sigmoid(5 (1 - F)) (classes.py:138-189), fp32, no autograd."""
-        _no_history(p, "occupancy")
+        _no_history(p, "occupancy", "  For an occupancy grid to differentiate through (any loss on voxels), use "
+                    "soft_occupancy(p).")
+        return Fn.field(p, self._n, self._step, self._z0, 1, 5.0)
+
+    def soft_occupancy(self, p):
+        """(B, n, n, n) fp32 occupancy sigmoid(5 (1 - F)), differentiable w.r.t. ``p`` (the reference's occupancy with
+        autograd history, classes.py:138-189): the same bits as ``occupancy``; its backward is one CUDA vector-Jacobian
+        product, so any loss on the grid (MSE or BCE against voxels, masks, per-voxel weights, a soft-volume term, sums
+        of these) can be trained through it.  When ground-truth parameters exist, ``self(true, pred)`` is cheaper: it is
+        fused into one walk and never holds a grid in memory.  Under torch.no_grad(), or for a ``p`` that does not
+        require grad, a plain tensor."""
+        args = (self._n, self._step, self._z0, 5.0)
+        if torch.is_grad_enabled() and isinstance(p, torch.Tensor) and p.requires_grad:
+            return Fn.OccupancyFn.apply(p, *args)
         return Fn.field(p, self._n, self._step, self._z0, 1, 5.0)
 
     def __call__(self, true, pred):

@@ -597,15 +597,17 @@ SQ_HD void acc_zero(Acc& a) {
 //   grad wrt q    = sum_ij dM_ij/dq * grad M_ij,  M = mat(conj(q))
 // z_is_index: the z moment gm[i][2] holds sum gs_i * cf (grid index units, column kernels) instead of
 // sum gs_i * (z - t_z) (point-list kernel).
+// z_centre (z_is_index only): the z moment holds sum gs_i * (cf - z_centre) instead (explicit_column's VJP mode: plane_of_t()).
 SQ_HD void finalize_sample(const SampleFull& S, const Grid& g, const double* acc, double scale, bool z_is_index,
-                           double* grad12) {
+                           double* grad12, double z_centre = 0.0) {
+    const double tz = z_centre != 0.0 ? S.t[2] - g.step * z_centre : S.t[2];
     const double* gs = acc; const double* gm = acc + 3; const double* wa = acc + 12; const double* ge = acc + 15;
     double gM[9];
     for (int i = 0; i < 3; ++i) {
         const double ia = S.ia[i];
         gM[3 * i + 0] = 2.0 * ia * gm[3 * i + 0];
         gM[3 * i + 1] = 2.0 * ia * gm[3 * i + 1];
-        gM[3 * i + 2] = 2.0 * ia * (z_is_index ? g.step * gm[3 * i + 2] - S.t[2] * gs[i] : gm[3 * i + 2]);
+        gM[3 * i + 2] = 2.0 * ia * (z_is_index ? g.step * gm[3 * i + 2] - tz * gs[i] : gm[3 * i + 2]);
     }
     for (int i = 0; i < 3; ++i) grad12[i] = -2.0 * wa[i] * S.ia[i] * S.mask[i] * scale;
     grad12[3] = kLn2 * ge[0] * S.mask[3] * scale;
@@ -648,6 +650,21 @@ constexpr float kImplicitCullBits = SQ_IMPLICIT_CULL_BITS;
 // |s_i| < bound24 the occupancy is < 2^-24 and is taken as 0 (DESIGN.md "culling").
 SQ_HD float cull_bound_bits(float kl, float bits) { return sqrtf((1.0f + bits / kl) * 1.002f); }
 SQ_HD float implicit_cull_bound(float kl) { return cull_bound_bits(kl, kImplicitCullBits); }
+
+// The VJP of the occupancy field (sq_occupancy_vjp) drops every point whose weight o (1 - o) is below 2^-bits: it culls the
+// walk at that level and cuts the backward there too.  Unlike the loss, whose upstream (o_p - o_t) vanishes where both
+// occupancies are tiny, an upstream can be large and of one sign over the whole soft shell (d sum(o) / d theta: the soft
+// volume), so what is dropped adds up coherently.  Per unit of grid volume that is
+//   sum_{x > bits} k 2^-x |dF/dtheta| dV  ~  2^-bits |dF/dtheta| dV/dF   (one octave of o (1 - o) spans ln2 / k in F)
+// at F_cut = 1 + bits ln2 / k, against the per-sample tolerance 5e-9 n^3 max|upstream|, i.e. 5e-9 per unit volume: the
+// grid size drops out and bits depends on k alone.  Measured at k = 5 on the host build (tests/emu/emu_occ_vjp.cpp, the
+// random goldens at R = 8..64, edge, pred24, zero planes), worst entry in units of the tolerance for the upstream +1 on
+// the shell o (1 - o) in [2^-34, 2^-20] -- one sign, all of it below the loss path's 2^-24:
+//   cut at 24 bits: 26..63    28: 1.5..5.6    32: 0.07..0.15    34 and beyond: < 1e-3 (the whole shell kept)
+// i.e. the dropped sum shrinks ~16x per 4 bits; at 36 bits what lies beyond the cut is ~1/100 of the tolerance for any
+// upstream.  (The constant upstream is not limited by the cut: from 28 bits on its error is the fp32 floor of the sums.)
+// A sharper sigmoid needs fewer bits (F_cut closer to 1), so 36 is conservative for k >= 5.
+constexpr float kExplicitVjpBits = 36.0f;
 
 // The box is loose for round shapes (for an ellipsoid it has twice the volume of the level set).  Second bound, from
 // the power-mean inequality (exponents 2/e >= 2):
@@ -1330,11 +1347,14 @@ __device__ __forceinline__ void forward_pair(const Sample& Sa, const Sample& Sb,
 }
 #endif
 
-// one z plane of explicit_column; HAS_T / HAS_P: whether the true / predicted SQ can be occupied on this plane
-template <bool BWD, bool HAS_T, bool HAS_P>
+// one z plane of explicit_column; HAS_T / HAS_P: whether the true / predicted SQ can be occupied on this plane.
+// VJP (sq_occupancy_vjp): no true SQ, no squared difference; the point's weight is the upstream voxel `up` (dL/d o) and the
+// weight cut is `kact` bits (kExplicitVjpBits) instead of kActiveExplicit, and the z moment is taken about plane `zc`.
+template <bool BWD, bool HAS_T, bool HAS_P, bool VJP = false>
 SQ_HD void explicit_step(const Sample& St, const Sample& Sp, float kl, float cf,
                          const float* bht, const float* blt, const float* bhp, const float* blp,
-                         float& sq, float* gs, float* gz, Acc& acc) {
+                         float& sq, float* gs, float* gz, Acc& acc, float up = 0.f, float kact = kActiveExplicit, float zc = 0.f) {
+    static_assert(!VJP || (BWD && !HAS_T && HAS_P), "the VJP mode walks the predicted SQ alone");
     float ot = 0.f, op = 0.f, xp = 1e30f, ep = 0.f;
     Fwd ft, fp;
 #if defined(__CUDA_ARCH__) && SQ_F32X2 && SQ_EXP_PAIR
@@ -1357,19 +1377,21 @@ SQ_HD void explicit_step(const Sample& St, const Sample& Sp, float kl, float cf,
     if (HAS_P) op = occupancy(fp.F, kl, xp, ep);
     }
     const float d = ot - op;
-    sq = fmaf(d, d, sq);
+    if (!VJP) sq = fmaf(d, d, sq);
     if (BWD && HAS_P) {
-        const bool active = fabsf(xp) < kActiveExplicit;
+        // VJP: points under a zero upstream voxel carry nothing (sparse upstreams skip the backward)
+        const bool active = VJP ? (fabsf(xp) < kact && up != 0.0f) : fabsf(xp) < kActiveExplicit;
         if (SQ_ANY(active)) {
             // d/dF_p of (o_t - o_p)^2 = 2 d * k o_p (1 - o_p); constants 2, k applied in finalize
-            const float W = active ? d * ep * op * op : 0.0f;
+            // (VJP: d o_p / dF_p = -k o_p (1 - o_p) times the upstream; -k applied in finalize)
+            const float W = active ? (VJP ? up : d) * ep * op * op : 0.0f;
             Fwd fa = fp;
             if (!active) fwd_neutral(fa);
             Bwd b;
             point_backward(fa, W, b);
             for (int i = 0; i < 3; ++i) {
                 gs[i] += b.gs[i];
-                gz[i] = fmaf(b.gs[i], cf, gz[i]);
+                gz[i] = fmaf(b.gs[i], VJP ? cf - zc : cf, gz[i]);
             }
             acc.ge[0] += b.ge[0];
             acc.ge[1] += b.ge[1];
@@ -1377,22 +1399,60 @@ SQ_HD void explicit_step(const Sample& St, const Sample& Sp, float kl, float cf,
     }
 }
 
-template <bool BWD>
+// The plane "index" of t_z, cf(t) = t_z / step, rounded to fp32 the same way in the column kernel and in finalize.  The
+// VJP's z moment is taken about it: sum gs (cf - cf(t)) instead of sum gs cf.  The gradient sums of a VJP can be large and of
+// one sign on each side of the object and cancel only between far-apart columns (the soft volume's rotation and translation
+// entries; measured: 1e-5 of the size entries), so their fp32 roundings have to be small against the centred moment, not
+// against z (t_z = 1: |z| up to 1, |z - t_z| at most ~0.35 over the object's shell).
+SQ_HD float plane_of_t(const Sample& S, const Grid& g) { return d2f(S.t[2] / g.step); }
+
+// read-only load of an upstream value (device: through the non-coherent path, cached in L1)
+SQ_HD float load_ro(const float* p) {
+#if defined(__CUDA_ARCH__)
+    return __ldg(p);
+#else
+    return *p;
+#endif
+}
+
+// VJP (sq_occupancy_vjp): the predicted SQ alone over rp (rt is ignored), every point weighted by the upstream voxel
+// up[c] of the column (NULL: a masked lane, weight 0), weight cut at `kact` bits, the z moment acc.gm[i][2] taken about
+// plane_of_t() (finalize_sample's z_centre); returns 0.
+// A lane reads its own column, consecutive floats along z, 32 different rows per warp and plane: each 32-byte sector
+// comes from DRAM once per walk and serves the next planes from L1.  The loads are issued two planes ahead of the plane
+// that uses them, so the one plane in eight that misses L1 waits behind two forward chains instead of stalling one.
+template <bool BWD, bool VJP = false>
 SQ_HD float explicit_column(const Sample& St, const Sample& Sp, const Grid& g, float kl,
                             const float* bht, const float* blt, const float* bhp, const float* blp,
-                            Range rt, Range rp, float dx, float dy, Acc& acc) {
+                            Range rt, Range rp, float dx, float dy, Acc& acc,
+                            const float* up = nullptr, float kact = kActiveExplicit) {
     float sq = 0.f;
     float gs[3] = {0.f, 0.f, 0.f}, gz[3] = {0.f, 0.f, 0.f};
-    const bool et = rt.hi < rt.lo, ep = rp.hi < rp.lo;
-    const int c_hi = rt.hi > rp.hi ? rt.hi : rp.hi;
-    const int c_lo = et ? rp.lo : ep ? rt.lo : (rt.lo < rp.lo ? rt.lo : rp.lo);
-    float cfi = (float)c_hi;
-    for (int c = c_hi; c >= c_lo; --c, cfi -= 1.0f) {
-        const float cf = (c == 0) ? Sp.cf0 : cfi;
-        const bool in_t = (c >= rt.lo && c <= rt.hi), in_p = (c >= rp.lo && c <= rp.hi);    // warp-uniform
-        if (in_t && in_p) explicit_step<BWD, true, true>(St, Sp, kl, cf, bht, blt, bhp, blp, sq, gs, gz, acc);
-        else if (in_p)    explicit_step<BWD, false, true>(St, Sp, kl, cf, bht, blt, bhp, blp, sq, gs, gz, acc);
-        else if (in_t)    explicit_step<BWD, true, false>(St, Sp, kl, cf, bht, blt, bhp, blp, sq, gs, gz, acc);
+    float zc = 0.f;
+    if constexpr (VJP) {
+        zc = plane_of_t(Sp, g);
+        const int c_hi = rp.hi, c_lo = rp.lo;
+        float u0 = (up && c_hi >= c_lo) ? load_ro(up + c_hi) : 0.f;
+        float u1 = (up && c_hi - 1 >= c_lo) ? load_ro(up + c_hi - 1) : 0.f;
+        float cfi = (float)c_hi;
+        for (int c = c_hi; c >= c_lo; --c, cfi -= 1.0f) {
+            const float u2 = (up && c - 2 >= c_lo) ? load_ro(up + c - 2) : 0.f;
+            const float cf = (c == 0) ? Sp.cf0 : cfi;
+            explicit_step<true, false, true, true>(Sp, Sp, kl, cf, bhp, blp, bhp, blp, sq, gs, gz, acc, u0, kact, zc);
+            u0 = u1; u1 = u2;
+        }
+    } else {
+        const bool et = rt.hi < rt.lo, ep = rp.hi < rp.lo;
+        const int c_hi = rt.hi > rp.hi ? rt.hi : rp.hi;
+        const int c_lo = et ? rp.lo : ep ? rt.lo : (rt.lo < rp.lo ? rt.lo : rp.lo);
+        float cfi = (float)c_hi;
+        for (int c = c_hi; c >= c_lo; --c, cfi -= 1.0f) {
+            const float cf = (c == 0) ? Sp.cf0 : cfi;
+            const bool in_t = (c >= rt.lo && c <= rt.hi), in_p = (c >= rp.lo && c <= rp.hi);    // warp-uniform
+            if (in_t && in_p) explicit_step<BWD, true, true>(St, Sp, kl, cf, bht, blt, bhp, blp, sq, gs, gz, acc);
+            else if (in_p)    explicit_step<BWD, false, true>(St, Sp, kl, cf, bht, blt, bhp, blp, sq, gs, gz, acc);
+            else if (in_t)    explicit_step<BWD, true, false>(St, Sp, kl, cf, bht, blt, bhp, blp, sq, gs, gz, acc);
+        }
     }
     if (BWD) {
         for (int i = 0; i < 3; ++i) {
@@ -1400,8 +1460,9 @@ SQ_HD float explicit_column(const Sample& St, const Sample& Sp, const Grid& g, f
             acc.gm[3 * i + 0] = fmaf(gs[i], dx, acc.gm[3 * i + 0]);
             acc.gm[3 * i + 1] = fmaf(gs[i], dy, acc.gm[3 * i + 1]);
             acc.gm[3 * i + 2] += gz[i];
-            // sum gs_i s_i with s_i = base_i + d_i cf (see implicit_column)
-            acc.wa[i] += fmaf(bhp[i], gs[i], fmaf(Sp.dh[i], gz[i], fmaf(blp[i], gs[i], Sp.dl[i] * gz[i])));
+            // sum gs_i s_i with s_i = base_i + d_i cf (see implicit_column; VJP: s_i = (base_i + d_i zc) + d_i (cf - zc))
+            if (VJP) acc.wa[i] += fmaf(fmaf(Sp.dh[i], zc, bhp[i]), gs[i], fmaf(Sp.dh[i], gz[i], fmaf(fmaf(Sp.dl[i], zc, blp[i]), gs[i], Sp.dl[i] * gz[i])));
+            else acc.wa[i] += fmaf(bhp[i], gs[i], fmaf(Sp.dh[i], gz[i], fmaf(blp[i], gs[i], Sp.dl[i] * gz[i])));
         }
     }
     return sq;

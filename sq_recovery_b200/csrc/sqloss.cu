@@ -559,6 +559,27 @@ __device__ __forceinline__ void warp_reduce_store(const Acc& a, float* tile, flo
     tile_reduce_store(tile, row);
 }
 
+// The same with the 32 lanes added in fp64 and the row rounded to fp32 once (the VJP kernel: its sums cancel only across rows,
+// so each row's rounding has to be as small as it can be).  Every row is written (there is no loss to tell empty ones by).
+__device__ __forceinline__ void warp_reduce_store_f64(const Acc& a, float* tile, float* row) {
+    const int lane = threadIdx.x & 31;
+    float v[kRedStride];
+    acc_to_array(a, v);
+    v[18] = v[19] = 0.f;
+    tile_put(tile, v);
+    __syncwarp();
+    if (lane < kRow) {
+        double s0 = 0.0, s1 = 0.0;
+#pragma unroll
+        for (int r = 0; r < 32; r += 2) {
+            s0 += (double)tile[r * kRedStride + lane];
+            s1 += (double)tile[(r + 1) * kRedStride + lane];
+        }
+        row[lane] = (float)(s0 + s1);
+    }
+    __syncwarp();
+}
+
 // per-thread Acc -> one row of kAccN floats per BLOCK (point-list kernel)
 __device__ __forceinline__ void block_reduce_store(const Acc& a, float (*red)[kAccN], float* row) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1170,6 +1191,64 @@ explicit_kernel(const SampleFull* __restrict__ tru, const SampleFull* __restrict
     retire(ctl, wp.joined, total_items, lane);
 }
 
+// Vector-Jacobian product of the occupancy field (sq_occupancy_vjp): explicit_kernel's work loop with the predicted SQ
+// alone and explicit_column's VJP mode -- the upstream voxels up[b][x][y][z] (sq_field's layout) weight the points, the cut is
+// `kact` bits, the walk covers the z range culled at the same level (`bound`).  A sibling kernel rather than a third
+// instantiation of explicit_kernel, so that the loss kernels keep their parameter lists and code.
+__global__ void __launch_bounds__(SQ_EXP_THREADS, SQ_EXP_MINB)
+explicit_vjp_kernel(const SampleFull* __restrict__ pred, Grid g, Layout L, float kl, float bound, float kact,
+                    const float* __restrict__ up, int total_items, Control* __restrict__ ctl, const int* __restrict__ queue,
+                    int cap, float* __restrict__ partials) {
+    __shared__ Sample Psh[SQ_EXP_THREADS / 32];
+    __shared__ __align__(16) float tiles[SQ_EXP_THREADS / 32][kRedFloats];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    Sample& Sp = Psh[warp];
+    WorkPipe wp;
+    wp.start(ctl, queue, cap, total_items, true, lane);      // proven-empty items are dropped (their rows: plan kernel)
+    {
+        SampleFetch pre_p;
+        if (wp.item >= 0) pre_p.fetch(pred + L.sample_of(wp.item), lane);
+        while (wp.item >= 0) {
+            const int item = wp.item;
+            int b, chunk;
+            L.split(item, b, chunk);
+            pre_p.commit(&Sp, lane);
+            Acc acc;
+            acc_zero(acc);
+            ColIter it;
+            it.init(L, chunk, lane);
+            for (int k = 0; k < L.cpt; ++k, it.next(L)) {
+                const bool valid = it.valid(L);
+                const int ia = valid ? it.ia : 0, ib = valid ? it.ib : 0;
+                float bhp[3], blp[3];
+                float dxy[2];
+                Range rp;
+                column_base_f32(Sp, g, ia, ib, bhp);
+                column_range(Sp, g, bound, bhp, rp.lo, rp.hi);
+                if (!valid) { rp.lo = 0; rp.hi = -1; }
+                warp_range(g.n, rp.lo, rp.hi);
+                if (rp.hi < rp.lo) continue;                                  // every point of the group below the cut
+                column_base(Sp, g, ia, ib, bhp, blp, dxy);
+                const float* col = valid ? up + (((size_t)b * g.n + ia) * g.n + ib) * g.n : nullptr;
+                Acc c;
+                acc_zero(c);
+                explicit_column<true, true>(Sp, Sp, g, kl, bhp, blp, bhp, blp, Range{0, -1}, rp, dxy[0], dxy[1], c, col, kact);
+                if (valid) {
+#pragma unroll
+                    for (int i = 0; i < 3; ++i) { acc.gs[i] += c.gs[i]; acc.wa[i] += c.wa[i]; }
+#pragma unroll
+                    for (int i = 0; i < 9; ++i) acc.gm[i] += c.gm[i];
+                    acc.ge[0] += c.ge[0]; acc.ge[1] += c.ge[1];
+                }
+            }
+            if (wp.claim(lane)) pre_p.fetch(pred + L.sample_of(wp.next), lane);
+            warp_reduce_store_f64(acc, tiles[warp], partials + (size_t)item * kRow);
+            wp.rotate();
+        }
+    }
+    retire(ctl, wp.joined, total_items, lane);
+}
+
 // ------------------------------------------------------------------------------------------------ IoU
 __global__ void __launch_bounds__(SQ_IOU_THREADS, SQ_IOU_MINB)
 iou_kernel(const SampleFull* __restrict__ tru, const SampleFull* __restrict__ pred, Grid g, Layout L, int total_items,
@@ -1302,7 +1381,7 @@ lsq_points_kernel(const SampleFull* __restrict__ samples, int chunks_per_sample,
 }
 
 // ------------------------------------------------------------------------------------------------ finalize
-enum { FIN_IMPLICIT = 0, FIN_EXPLICIT = 1, FIN_LSQ = 2 };
+enum { FIN_IMPLICIT = 0, FIN_EXPLICIT = 1, FIN_LSQ = 2, FIN_OCC_VJP = 3 };     // FIN_OCC_VJP: z moment about plane_of_t()
 
 // One block of kFinThreads per sample: every thread sums the partial rows r = t, t + kFinThreads, ... in fp64 (all loads
 // independent: one L2 round trip), a fixed-order tree (shuffles inside a warp, then the warps in index order) gives the
@@ -1382,7 +1461,7 @@ finalize_kernel(const SampleFull* __restrict__ samples, Grid g, int batch, int i
         }
     } else if (t == 0 && grad) {
         double gr[12];
-        finalize_sample(S, g, acc, grad_scale * vol, KIND != FIN_LSQ, gr);
+        finalize_sample(S, g, acc, grad_scale * vol, KIND != FIN_LSQ, gr, KIND == FIN_OCC_VJP ? (double)plane_of_t(S, g) : 0.0);
         if (KIND == FIN_LSQ)
             for (int i = 0; i < 3; ++i) gr[i] += S.mask[i] * (vol * S.ia[i]) * acc[17] * (0.5 * grad_scale);   // d (a1 a2 a3) / d a_i
         if (S.heads) heads_backward(S.hp, S.hrn, S.q, gr);
@@ -1781,6 +1860,38 @@ int sq_explicit_loss(const void* true_params, const void* pred, int params_dtype
         s.pred, g, batch, L.rows_per_sample, s.partials, (double)mult / n3,
         2.0 * (double)sharpness * (double)mult / (n3 * (double)batch), params_dtype, grad_pred, s.per_sample,
         per_sample, loss_out, &s.ctl->ticket, nullptr, queue ? s.item_class : nullptr);
+    SQ_TRY(cudaGetLastError());
+    return 0;
+}
+
+// plan (the predicted SQ alone, clamped, culled at the VJP's cut: proven-empty items carry no weight above the cut for any
+// upstream), the VJP column kernel, finalize with the scale of d o / d F = -k o (1 - o) alone.  Nothing is read that an
+// earlier call left behind.
+int sq_occupancy_vjp(const void* params, int params_dtype, int batch, int n, double step, double z0,
+                     float sharpness, const float* grad_field, void* grad_params,
+                     void* scratch, size_t scratch_bytes, sq_stream_t stream) {
+    Scratch s;
+    int rc = check_scratch(batch, n, scratch, scratch_bytes, &s);
+    if (rc) return rc;
+    if (!params || !grad_field || !grad_params) return (int)cudaErrorInvalidValue;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const Grid g = make_grid(n, step, z0);
+    const Layout L = make_layout(n, SQ_EXP_CPT);
+    const float kl = sharpness * kLog2e, kact = kExplicitVjpBits, bound = cull_bound_bits(kl, kact);
+    rc = launch_plan(params, nullptr, params_dtype, batch, true, g, L, bound, s, nullptr, s.item_class, nullptr, st);
+    if (rc) return rc;
+    const int items = batch * L.rows_per_sample;
+    const int* queue = L.rows_per_sample <= kPlanMaxItems ? s.queue : nullptr;
+    const int blocks = persistent_blocks(items, SQ_EXP_THREADS / 32, SQ_EXP_MINB);
+    {
+        ColumnKernelTimer timer(st);
+        explicit_vjp_kernel<<<blocks, SQ_EXP_THREADS, 0, st>>>(s.pred, g, L, kl, bound, kact, grad_field, items, s.ctl, queue,
+                                                               s.queue_cap, s.partials);
+    }
+    SQ_TRY(cudaGetLastError());
+    finalize_kernel<FIN_OCC_VJP><<<batch, kFinThreads, 0, st>>>(
+        s.pred, g, batch, L.rows_per_sample, s.partials, 0.0, -(double)sharpness, params_dtype, grad_params, s.per_sample,
+        nullptr, nullptr, &s.ctl->ticket, nullptr, queue ? s.item_class : nullptr);
     SQ_TRY(cudaGetLastError());
     return 0;
 }

@@ -384,6 +384,36 @@ def field(params: torch.Tensor, n: int, step: float, z0: float, mode: int, sharp
     return out
 
 
+class OccupancyFn(torch.autograd.Function):
+    """Differentiable ExplicitLoss.occupancy: the forward is the forward-only field (mode 1, same bits as ``field``); the
+    backward is the vector-Jacobian product kernel (sq_occupancy_vjp), which walks the grid again with the upstream voxels
+    as point weights.  Any loss on the occupancy grid can be trained through it; for the MSE against the occupancy of
+    known parameters the fused ExplicitLossFn is cheaper (no grid in memory, one walk)."""
+
+    @staticmethod
+    def forward(ctx, params, n, step, z0, sharpness):
+        _require_cuda(params, "params")
+        p, tag = _params(params)
+        ctx.p, ctx.tag, ctx.params_dtype = p, tag, params.dtype
+        ctx.args = (n, step, z0, sharpness)
+        return field(p, n, step, z0, 1, sharpness)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, go):
+        p, (n, step, z0, sharpness) = ctx.p, ctx.args
+        dev = p.device
+        B = p.shape[0]
+        g = go.float().contiguous()
+        grad = torch.empty_like(p)
+        scratch = _get_scratch(dev, B, n)
+        with _on_device(dev):
+            rc = _lib.lib().sq_occupancy_vjp(_ptr(p), ctx.tag, B, n, step, z0, sharpness, _ptr(g), _ptr(grad),
+                                             _ptr(scratch), scratch.numel(), _stream(dev))
+        _lib.check(rc, "sq_occupancy_vjp")
+        return grad.to(ctx.params_dtype), None, None, None, None
+
+
 class HostContext:
     """sq_ctx wrapper: the host-buffer entry points of the C ABI (what a non-torch caller binds)."""
 

@@ -2,7 +2,7 @@
 """Batched superquadric refinement by gradient descent -- the loop of torch/visu.py:120-186 without the GUI, run for
 thousands of SQs at once (SURVEY 8f-4).
 
-    python harness/optimize.py [--pairs 4096] [--steps 200] [--render 32] [--loss explicit|implicit|voxels]
+    python harness/optimize.py [--pairs 4096] [--steps 200] [--render 32] [--loss explicit|implicit|voxels|voxels-fused]
     python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 harness/optimize.py
 
 Per step and per SQ, exactly the reference's update (visu.py:176-186): params[:8] -= lr * grad[:8];
@@ -11,6 +11,8 @@ optimises ONE pair (batch 1); here every pair must see the gradient of ITS OWN l
 return is scaled back by the batch size.  Pairs are sharded over the ranks; no collective during the descent.
 --loss voxels fits to voxel data instead of ground-truth parameters: the target is the binarised occupancy
 (occupancy(true) > 0.5) on ExplicitLoss(R)'s grid, the criterion 100 mean((soft_occupancy(pred) - voxels)^2) (VoxelLoss).
+--loss voxels-fused is the same objective through ExplicitLoss.voxel_loss: the target is that grid as bool (read as bytes),
+loss and gradient are one fused walk, and no occupancy grid is held in memory.
 Prints one JSON line on rank 0: steps/s, loss evaluations (grid points) per second, IoU(128) before / after.
 """
 import argparse
@@ -69,7 +71,7 @@ def main():
     ap.add_argument("--pairs", type=int, default=4096)
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--render", type=int, default=32)
-    ap.add_argument("--loss", default="explicit", choices=["explicit", "implicit", "voxels"])
+    ap.add_argument("--loss", default="explicit", choices=["explicit", "implicit", "voxels", "voxels-fused"])
     args = ap.parse_args()
     import sq_recovery_b200 as S
     from sq_recovery_b200 import distributed as D
@@ -89,6 +91,9 @@ def main():
     elif args.loss == "voxels":
         grid = S.ExplicitLoss(R, dev)
         crit, target, pts = VoxelLoss(grid.soft_occupancy), voxelize(grid, true), (b1 - b0) * grid._n ** 3
+    elif args.loss == "voxels-fused":
+        grid = S.ExplicitLoss(R, dev)
+        crit, target, pts = grid.voxel_loss, voxelize(grid, true).bool(), (b1 - b0) * grid._n ** 3
     else:
         crit = S.ImplicitLoss(R, dev, 1.5, 260)
         target = S.ImplicitLoss(256, dev, 1.5, 260).depth_projection(true).unsqueeze(1).contiguous()

@@ -26,7 +26,7 @@ extern "C" {
 #endif
 
 typedef void* sq_stream_t;           /* cudaStream_t */
-enum { SQ_F32 = 0, SQ_F64 = 1, SQ_U8 = 2 };   /* SQ_U8: 8-bit depth images of the host-buffer calls only */
+enum { SQ_F32 = 0, SQ_F64 = 1, SQ_U8 = 2 };   /* SQ_U8: 8-bit depth images of the host-buffer calls, 8-bit voxels */
 
 /* Library / device introspection. */
 const char* sq_version(void);
@@ -150,6 +150,22 @@ int sq_field(const void* params, int params_dtype, int batch, int n, double step
 int sq_occupancy_vjp(const void* params, int params_dtype, int batch, int n, double step, double z0,
                      float sharpness, const float* grad_field, void* grad_params,
                      void* scratch, size_t scratch_bytes, sq_stream_t stream);
+
+/* ExplicitLoss's MSE of the occupancy field against voxel data (torch/classes.py:138-189), forward and backward in one
+ * walk, with no field in memory:
+ *   loss = mean_b mult * mean_vox (v - o_pred)^2,  o = sigmoid(sharpness (1 - F)), clamp and zero fix-up as in the loss,
+ *   v = voxel_scale * voxels[b][x][y][z]   (voxels: [batch,n,n,n] contiguous, index order [x][y][z], SQ_F32 or SQ_U8)
+ *   loss_out    [1] fp64 (may be NULL);  per_sample [batch] fp64 mult * mean_vox (v - o_pred)^2 (may be NULL)
+ *   grad_pred   [batch,12] d loss_out / d pred (params_dtype)          (NULL = forward only; the loss bits are the same)
+ * Same scratch contract as the other entry points; asynchronous on `stream`; self-contained.  Every voxel is read once
+ * and every one counts: where the predicted occupancy is below the cut, the term is v^2.  The walk and the backward cut
+ * are those of sq_occupancy_vjp (o (1 - o) < 2^-36: the difference v - o can be large and of one sign over the whole soft
+ * shell).  A NULL voxels or pred, or another voxel_dtype, returns cudaErrorInvalidValue.
+ */
+int sq_voxel_loss(const void* voxels, int voxel_dtype, float voxel_scale,
+                  const void* pred, int params_dtype, int batch, int n, double step, double z0,
+                  float sharpness, float mult, double* loss_out, double* per_sample, void* grad_pred,
+                  void* scratch, size_t scratch_bytes, sq_stream_t stream);
 
 /* ---- host-buffer entry points (what a non-torch caller binds; H2D/D2H copies happen inside) -------------------
  * An sq_ctx owns a stream, device buffers and pinned staging buffers on one device; buffers grow on demand and are

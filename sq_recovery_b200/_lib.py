@@ -28,6 +28,8 @@ _PROTOS = {
                                         c_void_p, c_void_p, c_size_t, c_void_p]),
     "sq_occupancy_vjp": (c_int, [c_void_p, c_int, c_int, c_int, c_double, c_double, c_float, c_void_p, c_void_p, c_void_p,
                                  c_size_t, c_void_p]),
+    "sq_voxel_loss": (c_int, [c_void_p, c_int, c_float, c_void_p, c_int, c_int, c_int, c_double, c_double, c_float, c_float,
+                              c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "sq_explicit_loss": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_double, c_float, c_float,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "sq_iou_counts": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_double, c_void_p, c_void_p,

@@ -104,6 +104,20 @@ class ExplicitLoss(_GridLoss):
     def __call__(self, true, pred):
         return Fn.ExplicitLossFn.apply(true, pred, self._n, self._step, self._z0, 5.0, 100.0, torch.is_grad_enabled())
 
+    def voxel_loss(self, voxels, pred, voxel_scale=None):
+        """0-dim fp64 loss 100 mean((occupancy(pred) - v)^2), averaged over the batch like ``self(true, pred)``, against
+        voxel data instead of true parameters: the reference's objective with the target occupancy replaced by voxels.
+        ``voxels`` is (B, n, n, n) on this loss's grid, index order [x][y][z], on ``pred``'s device: float32 (float64 is
+        rounded to it), bool, or uint8 read as v = voxel_scale * byte (default 1/255).  Forward and backward are one CUDA
+        walk; no occupancy grid is held in memory, and 8-bit voxels are read as bytes.  The gradient reaches ``pred``
+        only: for a loss that must differentiate the voxels too, use soft_occupancy(pred)."""
+        if torch.is_grad_enabled() and isinstance(voxels, torch.Tensor) and voxels.requires_grad:
+            raise RuntimeError(
+                "sq_recovery_b200: voxel_loss() gives a gradient for pred only, and it was given voxels that require grad. "
+                "Pass voxels.detach(), or build the loss from soft_occupancy(pred), which differentiates any loss on the grid.")
+        return Fn.VoxelLossFn.apply(voxels, pred, self._n, self._step, self._z0, 5.0, 100.0, voxel_scale,
+                                    torch.is_grad_enabled())
+
 
 class ImplicitLoss(_GridLoss):
     """MAE between the input depth image and a soft depth render of the predicted SQ (torch/classes.py:203-295)."""

@@ -1350,11 +1350,14 @@ __device__ __forceinline__ void forward_pair(const Sample& Sa, const Sample& Sb,
 // one z plane of explicit_column; HAS_T / HAS_P: whether the true / predicted SQ can be occupied on this plane.
 // VJP (sq_occupancy_vjp): no true SQ, no squared difference; the point's weight is the upstream voxel `up` (dL/d o) and the
 // weight cut is `kact` bits (kExplicitVjpBits) instead of kActiveExplicit, and the z moment is taken about plane `zc`.
-template <bool BWD, bool HAS_T, bool HAS_P, bool VJP = false>
+// VOX (with VJP; sq_voxel_loss): `up` is the target voxel v and takes the place of o_t: d = v - o_p, sq += d^2, weight d as in
+// the loss, with the VJP's cut and z centre.  BWD = false is the forward-only walk of the same points.
+template <bool BWD, bool HAS_T, bool HAS_P, bool VJP = false, bool VOX = false>
 SQ_HD void explicit_step(const Sample& St, const Sample& Sp, float kl, float cf,
                          const float* bht, const float* blt, const float* bhp, const float* blp,
                          float& sq, float* gs, float* gz, Acc& acc, float up = 0.f, float kact = kActiveExplicit, float zc = 0.f) {
-    static_assert(!VJP || (BWD && !HAS_T && HAS_P), "the VJP mode walks the predicted SQ alone");
+    static_assert(!VJP || ((BWD || VOX) && !HAS_T && HAS_P), "the VJP mode walks the predicted SQ alone");
+    static_assert(!VOX || VJP, "the voxel loss is a variant of the VJP walk");
     float ot = 0.f, op = 0.f, xp = 1e30f, ep = 0.f;
     Fwd ft, fp;
 #if defined(__CUDA_ARCH__) && SQ_F32X2 && SQ_EXP_PAIR
@@ -1376,15 +1379,15 @@ SQ_HD void explicit_step(const Sample& St, const Sample& Sp, float kl, float cf,
     if (HAS_T) { float xt, et; ot = occupancy(ft.F, kl, xt, et); }
     if (HAS_P) op = occupancy(fp.F, kl, xp, ep);
     }
-    const float d = ot - op;
-    if (!VJP) sq = fmaf(d, d, sq);
+    const float d = (VOX ? up : ot) - op;
+    if (!VJP || VOX) sq = fmaf(d, d, sq);
     if (BWD && HAS_P) {
         // VJP: points under a zero upstream voxel carry nothing (sparse upstreams skip the backward)
-        const bool active = VJP ? (fabsf(xp) < kact && up != 0.0f) : fabsf(xp) < kActiveExplicit;
+        const bool active = VJP ? (fabsf(xp) < kact && (VOX || up != 0.0f)) : fabsf(xp) < kActiveExplicit;
         if (SQ_ANY(active)) {
             // d/dF_p of (o_t - o_p)^2 = 2 d * k o_p (1 - o_p); constants 2, k applied in finalize
             // (VJP: d o_p / dF_p = -k o_p (1 - o_p) times the upstream; -k applied in finalize)
-            const float W = active ? (VJP ? up : d) * ep * op * op : 0.0f;
+            const float W = active ? (VJP && !VOX ? up : d) * ep * op * op : 0.0f;
             Fwd fa = fp;
             if (!active) fwd_neutral(fa);
             Bwd b;
@@ -1414,33 +1417,60 @@ SQ_HD float load_ro(const float* p) {
     return *p;
 #endif
 }
+SQ_HD float load_ro(const unsigned char* p) {
+#if defined(__CUDA_ARCH__)
+    return (float)__ldg(p);
+#else
+    return (float)*p;
+#endif
+}
+
+// sum of v^2, v = vscale * vox[c], over the planes of one column of n voxels outside the walked range rp (all of them when
+// rp is empty): the voxel loss's terms where the predicted occupancy is below the cut and taken as 0.  NULL: a masked lane.
+// No MUFU work: the loop is bound by the loads, which are independent of each other.
+template <typename V>
+SQ_HD float voxel_sq_outside(const V* vox, int n, Range rp, float vscale) {
+    float sq = 0.f;
+    if (!vox) return sq;
+    const int hi = rp.hi < rp.lo ? -1 : rp.hi, lo = rp.hi < rp.lo ? 0 : rp.lo;
+#pragma unroll 4
+    for (int c = hi + 1; c < n; ++c) { const float v = vscale * load_ro(vox + c); sq = fmaf(v, v, sq); }
+#pragma unroll 4
+    for (int c = 0; c < lo; ++c) { const float v = vscale * load_ro(vox + c); sq = fmaf(v, v, sq); }
+    return sq;
+}
 
 // VJP (sq_occupancy_vjp): the predicted SQ alone over rp (rt is ignored), every point weighted by the upstream voxel
 // up[c] of the column (NULL: a masked lane, weight 0), weight cut at `kact` bits, the z moment acc.gm[i][2] taken about
 // plane_of_t() (finalize_sample's z_centre); returns 0.
+// VOX (with VJP; sq_voxel_loss): up[c] (V = float or uint8_t, times vscale) is the target voxel v; returns the column's
+// whole sum of squares: (v - o_p)^2 over the walked planes, then v^2 over the others (voxel_sq_outside).  With BWD = false
+// the same planes are walked for the loss alone, so the loss does not depend on whether a gradient is asked for.
 // A lane reads its own column, consecutive floats along z, 32 different rows per warp and plane: each 32-byte sector
 // comes from DRAM once per walk and serves the next planes from L1.  The loads are issued two planes ahead of the plane
 // that uses them, so the one plane in eight that misses L1 waits behind two forward chains instead of stalling one.
-template <bool BWD, bool VJP = false>
+template <bool BWD, bool VJP = false, bool VOX = false, typename V = float>
 SQ_HD float explicit_column(const Sample& St, const Sample& Sp, const Grid& g, float kl,
                             const float* bht, const float* blt, const float* bhp, const float* blp,
                             Range rt, Range rp, float dx, float dy, Acc& acc,
-                            const float* up = nullptr, float kact = kActiveExplicit) {
+                            const V* up = nullptr, float kact = kActiveExplicit, float vscale = 1.f) {
     float sq = 0.f;
     float gs[3] = {0.f, 0.f, 0.f}, gz[3] = {0.f, 0.f, 0.f};
     float zc = 0.f;
     if constexpr (VJP) {
         zc = plane_of_t(Sp, g);
         const int c_hi = rp.hi, c_lo = rp.lo;
-        float u0 = (up && c_hi >= c_lo) ? load_ro(up + c_hi) : 0.f;
-        float u1 = (up && c_hi - 1 >= c_lo) ? load_ro(up + c_hi - 1) : 0.f;
+        auto ld = [&](int c) { return VOX ? vscale * load_ro(up + c) : load_ro(up + c); };
+        float u0 = (up && c_hi >= c_lo) ? ld(c_hi) : 0.f;
+        float u1 = (up && c_hi - 1 >= c_lo) ? ld(c_hi - 1) : 0.f;
         float cfi = (float)c_hi;
         for (int c = c_hi; c >= c_lo; --c, cfi -= 1.0f) {
-            const float u2 = (up && c - 2 >= c_lo) ? load_ro(up + c - 2) : 0.f;
+            const float u2 = (up && c - 2 >= c_lo) ? ld(c - 2) : 0.f;
             const float cf = (c == 0) ? Sp.cf0 : cfi;
-            explicit_step<true, false, true, true>(Sp, Sp, kl, cf, bhp, blp, bhp, blp, sq, gs, gz, acc, u0, kact, zc);
+            explicit_step<BWD, false, true, true, VOX>(Sp, Sp, kl, cf, bhp, blp, bhp, blp, sq, gs, gz, acc, u0, kact, zc);
             u0 = u1; u1 = u2;
         }
+        if constexpr (VOX) sq += voxel_sq_outside(up, g.n, rp, vscale);
     } else {
         const bool et = rt.hi < rt.lo, ep = rp.hi < rp.lo;
         const int c_hi = rt.hi > rp.hi ? rt.hi : rp.hi;

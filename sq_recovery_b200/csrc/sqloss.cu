@@ -1249,6 +1249,76 @@ explicit_vjp_kernel(const SampleFull* __restrict__ pred, Grid g, Layout L, float
     retire(ctl, wp.joined, total_items, lane);
 }
 
+// MSE of the occupancy field against voxel data (sq_voxel_loss): explicit_vjp_kernel's work loop with explicit_column's VOX
+// mode -- the voxels vox[b][x][y][z] (V = float or uint8_t, times vscale) take the place of the upstream and of o_t.  Every
+// voxel counts, including those the walk never visits, so no item and no column is skipped: a column group whose warp range
+// is empty, and every column of an item the plan kernel proved empty (its Sample is not even fetched), adds its sum of v^2
+// (voxel_sq_outside).  All terms are non-negative and each voxel is read once.  BWD = false: the same walk, loss only.
+template <bool BWD, typename V>
+__global__ void __launch_bounds__(SQ_EXP_THREADS, SQ_EXP_MINB)
+explicit_vox_kernel(const SampleFull* __restrict__ pred, Grid g, Layout L, float kl, float bound, float kact,
+                    const V* __restrict__ vox, float vscale, int total_items, Control* __restrict__ ctl,
+                    const int* __restrict__ queue, int cap, float* __restrict__ partials) {
+    __shared__ Sample Psh[SQ_EXP_THREADS / 32];
+    __shared__ __align__(16) float tiles[SQ_EXP_THREADS / 32][kRedFloats];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    Sample& Sp = Psh[warp];
+    WorkPipe wp;
+    wp.start(ctl, queue, cap, total_items, false, lane);     // proven-empty items too: their voxels still count
+    {
+        SampleFetch pre_p;
+        if (wp.item >= 0) pre_p.fetch(pred + L.sample_of(wp.item), lane);
+        while (wp.item >= 0) {
+            const int item = wp.item;
+            const bool empty = wp.item_pos >= wp.empty_from;            // warp-uniform; Sp is stale then and never read
+            int b, chunk;
+            L.split(item, b, chunk);
+            pre_p.commit(&Sp, lane);
+            Acc acc;
+            acc_zero(acc);
+            ColIter it;
+            it.init(L, chunk, lane);
+            for (int k = 0; k < L.cpt; ++k, it.next(L)) {
+                const bool valid = it.valid(L);
+                const int ia = valid ? it.ia : 0, ib = valid ? it.ib : 0;
+                float bhp[3], blp[3];
+                float dxy[2];
+                Range rp{0, -1};
+                if (!empty) {
+                    column_base_f32(Sp, g, ia, ib, bhp);
+                    column_range(Sp, g, bound, bhp, rp.lo, rp.hi);
+                    if (!valid) { rp.lo = 0; rp.hi = -1; }
+                    warp_range(g.n, rp.lo, rp.hi);
+                }
+                const V* col = valid ? vox + (((size_t)b * g.n + ia) * g.n + ib) * g.n : nullptr;
+                if (rp.hi < rp.lo) {                                     // every point of the group below the cut
+                    acc.loss += voxel_sq_outside(col, g.n, rp, vscale);
+                    continue;
+                }
+                column_base(Sp, g, ia, ib, bhp, blp, dxy);
+                Acc c;
+                acc_zero(c);
+                const float sq = explicit_column<BWD, true, true>(Sp, Sp, g, kl, bhp, blp, bhp, blp, Range{0, -1}, rp, dxy[0],
+                                                                  dxy[1], c, col, kact, vscale);
+                if (valid) {
+                    acc.loss += sq;
+                    if (BWD) {
+#pragma unroll
+                        for (int i = 0; i < 3; ++i) { acc.gs[i] += c.gs[i]; acc.wa[i] += c.wa[i]; }
+#pragma unroll
+                        for (int i = 0; i < 9; ++i) acc.gm[i] += c.gm[i];
+                        acc.ge[0] += c.ge[0]; acc.ge[1] += c.ge[1];
+                    }
+                }
+            }
+            if (wp.claim(lane)) pre_p.fetch(pred + L.sample_of(wp.next), lane);
+            warp_reduce_store_f64(acc, tiles[warp], partials + (size_t)item * kRow);
+            wp.rotate();
+        }
+    }
+    retire(ctl, wp.joined, total_items, lane);
+}
+
 // ------------------------------------------------------------------------------------------------ IoU
 __global__ void __launch_bounds__(SQ_IOU_THREADS, SQ_IOU_MINB)
 iou_kernel(const SampleFull* __restrict__ tru, const SampleFull* __restrict__ pred, Grid g, Layout L, int total_items,
@@ -1382,6 +1452,7 @@ lsq_points_kernel(const SampleFull* __restrict__ samples, int chunks_per_sample,
 
 // ------------------------------------------------------------------------------------------------ finalize
 enum { FIN_IMPLICIT = 0, FIN_EXPLICIT = 1, FIN_LSQ = 2, FIN_OCC_VJP = 3 };     // FIN_OCC_VJP: z moment about plane_of_t()
+                                                                               // (sq_occupancy_vjp and sq_voxel_loss)
 
 // One block of kFinThreads per sample: every thread sums the partial rows r = t, t + kFinThreads, ... in fp64 (all loads
 // independent: one L2 round trip), a fixed-order tree (shuffles inside a warp, then the warps in index order) gives the
@@ -1892,6 +1963,51 @@ int sq_occupancy_vjp(const void* params, int params_dtype, int batch, int n, dou
     finalize_kernel<FIN_OCC_VJP><<<batch, kFinThreads, 0, st>>>(
         s.pred, g, batch, L.rows_per_sample, s.partials, 0.0, -(double)sharpness, params_dtype, grad_params, s.per_sample,
         nullptr, nullptr, &s.ctl->ticket, nullptr, queue ? s.item_class : nullptr);
+    SQ_TRY(cudaGetLastError());
+    return 0;
+}
+
+// plan (the predicted SQ alone, culled at the VJP's cut), the voxel column kernel, finalize with sq_explicit_loss's scales
+// and the VJP's z centre.  Finalize reads every item's row: the column kernel writes one for proven-empty items too.
+int sq_voxel_loss(const void* voxels, int voxel_dtype, float voxel_scale,
+                  const void* pred, int params_dtype, int batch, int n, double step, double z0,
+                  float sharpness, float mult, double* loss_out, double* per_sample, void* grad_pred,
+                  void* scratch, size_t scratch_bytes, sq_stream_t stream) {
+    Scratch s;
+    int rc = check_scratch(batch, n, scratch, scratch_bytes, &s);
+    if (rc) return rc;
+    if (!voxels || !pred || (voxel_dtype != SQ_F32 && voxel_dtype != SQ_U8)) return (int)cudaErrorInvalidValue;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const Grid g = make_grid(n, step, z0);
+    const Layout L = make_layout(n, SQ_EXP_CPT);
+    const float kl = sharpness * kLog2e, kact = kExplicitVjpBits, bound = cull_bound_bits(kl, kact);
+    rc = launch_plan(pred, nullptr, params_dtype, batch, true, g, L, bound, s, nullptr, s.item_class, nullptr, st);
+    if (rc) return rc;
+    const int items = batch * L.rows_per_sample;
+    const int* queue = L.rows_per_sample <= kPlanMaxItems ? s.queue : nullptr;
+    const int blocks = persistent_blocks(items, SQ_EXP_THREADS / 32, SQ_EXP_MINB);
+    {
+        ColumnKernelTimer timer(st);
+        const float* vf = static_cast<const float*>(voxels);
+        const uint8_t* vb = static_cast<const uint8_t*>(voxels);
+        if (voxel_dtype == SQ_U8) {
+            if (grad_pred) explicit_vox_kernel<true, uint8_t><<<blocks, SQ_EXP_THREADS, 0, st>>>(
+                s.pred, g, L, kl, bound, kact, vb, voxel_scale, items, s.ctl, queue, s.queue_cap, s.partials);
+            else explicit_vox_kernel<false, uint8_t><<<blocks, SQ_EXP_THREADS, 0, st>>>(
+                s.pred, g, L, kl, bound, kact, vb, voxel_scale, items, s.ctl, queue, s.queue_cap, s.partials);
+        } else {
+            if (grad_pred) explicit_vox_kernel<true, float><<<blocks, SQ_EXP_THREADS, 0, st>>>(
+                s.pred, g, L, kl, bound, kact, vf, voxel_scale, items, s.ctl, queue, s.queue_cap, s.partials);
+            else explicit_vox_kernel<false, float><<<blocks, SQ_EXP_THREADS, 0, st>>>(
+                s.pred, g, L, kl, bound, kact, vf, voxel_scale, items, s.ctl, queue, s.queue_cap, s.partials);
+        }
+    }
+    SQ_TRY(cudaGetLastError());
+    const double n3 = (double)n * n * n;
+    finalize_kernel<FIN_OCC_VJP><<<batch, kFinThreads, 0, st>>>(
+        s.pred, g, batch, L.rows_per_sample, s.partials, (double)mult / n3,
+        2.0 * (double)sharpness * (double)mult / (n3 * (double)batch), params_dtype, grad_pred, s.per_sample,
+        per_sample, loss_out, &s.ctl->ticket, nullptr, nullptr);
     SQ_TRY(cudaGetLastError());
     return 0;
 }

@@ -414,6 +414,53 @@ class OccupancyFn(torch.autograd.Function):
         return grad.to(ctx.params_dtype), None, None, None, None
 
 
+def _voxels(voxels: torch.Tensor, B: int, n: int, voxel_scale: Optional[float]) -> Tuple[torch.Tensor, int, float]:
+    """Contiguous voxel grid, its dtype tag and scale: float32 as is, float64 as float32, bool as bytes with scale 1,
+    uint8 with scale 1/255 (the convention of 8-bit depth images) unless `voxel_scale` says otherwise."""
+    if voxels.shape != (B, n, n, n):
+        raise ValueError(f"expected voxels of shape {(B, n, n, n)} (B, n, n, n) on this loss's grid, got {tuple(voxels.shape)}")
+    if voxel_scale is not None and voxels.dtype != torch.uint8:
+        raise ValueError(f"voxel_scale applies to uint8 voxels only (got {voxels.dtype})")
+    if voxels.dtype == torch.uint8:
+        return voxels.contiguous(), _lib.SQ_U8, float(voxel_scale) if voxel_scale is not None else 1.0 / 255.0
+    if voxels.dtype == torch.bool:
+        return voxels.contiguous().view(torch.uint8), _lib.SQ_U8, 1.0
+    return voxels.float().contiguous(), _lib.SQ_F32, 1.0
+
+
+class VoxelLossFn(torch.autograd.Function):
+    """ExplicitLoss.voxel_loss: mult * mean((occupancy(pred) - voxels)^2) per sample, averaged over the batch, forward and
+    backward in one walk (sq_voxel_loss); no occupancy grid is held in memory.  The gradient reaches ``pred`` only."""
+
+    @staticmethod
+    def forward(ctx, voxels, pred, n, step, z0, sharpness, mult, voxel_scale=None, grad_mode=True):
+        _require_cuda(pred, "pred"); _require_cuda(voxels, "voxels")
+        dev = pred.device
+        if voxels.device != dev:
+            raise ValueError(f"voxels ({voxels.device}) must be on pred's device ({dev})")
+        p, tag = _params(pred)
+        B = p.shape[0]
+        v, vtag, scale = _voxels(voxels, B, n, voxel_scale)
+        loss = torch.empty((), dtype=torch.float64, device=dev)
+        grad = torch.empty_like(p) if (grad_mode and ctx.needs_input_grad[1]) else None
+        scratch = _get_scratch(dev, B, n)
+        with _on_device(dev):
+            rc = _lib.lib().sq_voxel_loss(_ptr(v), vtag, scale, _ptr(p), tag, B, n, step, z0, sharpness, mult, _ptr(loss),
+                                          None, _ptr(grad), _ptr(scratch), scratch.numel(), _stream(dev))
+        _lib.check(rc, "sq_voxel_loss")
+        ctx.grad = grad
+        ctx.pred_dtype = pred.dtype
+        return loss
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, go):
+        g = None
+        if ctx.grad is not None:
+            g = (ctx.grad * go).to(ctx.pred_dtype)
+        return None, g, None, None, None, None, None, None, None
+
+
 class HostContext:
     """sq_ctx wrapper: the host-buffer entry points of the C ABI (what a non-torch caller binds)."""
 

@@ -131,6 +131,28 @@ int sq_least_squares_points(const void* pred, int pred_dtype, int batch, const f
                             double* loss_out, double* per_sample, void* grad_pred,
                             void* scratch, size_t scratch_bytes, sq_stream_t stream);
 
+/* Gauss-Newton normal equations of LeastSquares: per sample b, with residuals r_i = sqrt(a1 a2 a3) (F(x_i) - 1) over the
+ * sample's points and J_b their Jacobian (rows dr_i / dpred[b]), and no 1 / batch factor:
+ *   per_sample  [batch] fp64 E_b = sum_i r_i^2                 (the bits of sq_least_squares_points' / sq_least_squares' per_sample)
+ *   grad_pred   [batch,12] dE_b / dpred[b] = 2 J_b^T r_b (pred_dtype; the bits of sq_least_squares_points' grad_pred)
+ *   jtj         [batch,12,12] fp64 J_b^T J_b, row-major, exactly symmetric
+ * J carries the clamp masks as the gradient does (a clamped-out parameter has an exactly zero row and column of jtj), the
+ * quaternion is not normalised, and a point whose F >= 1e18 adds nothing to jtj (as it adds nothing to the gradient).
+ * Points and their addressing are those of sq_least_squares (the image call) and sq_least_squares_points (the list call).
+ * A NULL per_sample, grad_pred or jtj returns cudaErrorInvalidValue.  Scratch: sq_normal_scratch_bytes(batch, max_points),
+ * with max_points = render_size * render_size for the image call; the control-block contract is that of
+ * sq_scratch_bytes.  Asynchronous on `stream`, self-contained, and capturable into a CUDA graph.
+ */
+size_t sq_normal_scratch_bytes(int batch, long long max_points);
+int sq_least_squares_normal(const void* pred, int pred_dtype, int batch, int render_size,
+                            const float* target, long long target_stride_b, const int* row_off, const int* col_off,
+                            double* per_sample, void* grad_pred, double* jtj,
+                            void* scratch, size_t scratch_bytes, sq_stream_t stream);
+int sq_least_squares_points_normal(const void* pred, int pred_dtype, int batch, const float* points, long long stride,
+                                   const long long* offsets, long long max_points,
+                                   double* per_sample, void* grad_pred, double* jtj,
+                                   void* scratch, size_t scratch_bytes, sq_stream_t stream);
+
 /* ExplicitLoss.occupancy / IoUAccuracy.ins_outs (torch/classes.py:138-189, 394-426): the full field [batch,n,n,n]
  * (index order [x][y][z], fp32).  mode 0: F without clamp/fix-up (ins_outs); mode 1: sigmoid(sharpness (1-F))
  * with clamp and fix-up (occupancy).  A convenience for callers that want the grid itself.

@@ -39,6 +39,11 @@ _PROTOS = {
     "sq_points_scratch_bytes": (c_size_t, [c_int, c_longlong]),
     "sq_least_squares_points": (c_int, [c_void_p, c_int, c_int, c_void_p, c_longlong, c_void_p, c_longlong, c_void_p,
                                         c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "sq_normal_scratch_bytes": (c_size_t, [c_int, c_longlong]),
+    "sq_least_squares_normal": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_longlong, c_void_p, c_void_p, c_void_p,
+                                        c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "sq_least_squares_points_normal": (c_int, [c_void_p, c_int, c_int, c_void_p, c_longlong, c_void_p, c_longlong, c_void_p,
+                                               c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "sq_field": (c_int, [c_void_p, c_int, c_int, c_int, c_double, c_double, c_int, c_float, c_void_p, c_void_p,
                          c_size_t, c_void_p]),
     "sq_ctx_create": (c_int, [c_int, POINTER(c_void_p)]),

@@ -177,6 +177,19 @@ class LeastSquares(_GridLoss):
     def __call__(self, true, pred):
         return Fn.LeastSquaresFn.apply(true, pred, int(self.render_size), torch.is_grad_enabled())
 
+    def normal_equations(self, true, pred):
+        """Gauss-Newton normal equations of each sample's energy on the points of the (B, 1, H, W) depth images of
+        ``self(true, pred)``: ``(energy (B,) fp64, grad (B, 12) in pred's dtype, jtj (B, 12, 12) fp64)`` with
+        energy_b = sum_i r_i^2, r_i = sqrt(a1 a2 a3) (F(x_i) - 1), grad_b = d energy_b / d pred_b = 2 J_b^T r_b and
+        jtj_b = J_b^T J_b -- what a Levenberg-Marquardt step needs, from one walk over the points.  No 1 / B factor, no
+        autograd history (pred is read detached); clamped-out parameters have zero rows and columns in jtj."""
+        return Fn.lsq_normal_equations(true, pred, int(self.render_size))
+
+    def normal_equations_points(self, batch_points, params):
+        """``normal_equations`` on the (3, m_i) point lists of ``energy_function``: its energies, their gradients and
+        J^T J per sample, bit for bit the energies and gradients of ``energy_function``."""
+        return Fn.lsq_points_normal_equations(batch_points, params)
+
 
 class IoUAccuracy(_GridLoss):
     """IoU of the binarised (F <= 1) grids of true and predicted parameters (torch/classes.py:374-447)."""

@@ -1571,12 +1571,48 @@ SQ_HD void iou_column(const Sample& St, const Sample& Sp, const SampleFull* Ft, 
     }
 }
 
+// ---------------------------------------------------------------- LeastSquares: normal equations
+// Residual of one point r = sqrt(a1 a2 a3) (F - 1).  Its Jacobian row without the sqrt(a1 a2 a3) factor is
+//   j = dF/dtheta + (F - 1) d ln sqrt(a1 a2 a3) / dtheta = dF/dtheta + (F - 1) / (2 a_i)   (a_i entries only)
+// with dF/dtheta the per-point form of finalize_sample() at weight 1 (no clamp masks: finalize zeroes whole rows and
+// columns of J^T J).  JacConst holds the fp32 per-sample constants it needs; the 78 upper-triangle entries of j j^T are
+// summed per thread, in the order (0,0), (0,1) ... (0,11), (1,1) ... (11,11).
+constexpr int kJtJN = 78;
+struct JacConst {
+    float Ms[9];              // Ms (rows of M / a_i)
+    float ia[3];              // 1 / a_i
+    float q[4];               // raw quaternion (x, y, z, w)
+};
+SQ_HD void jac_const(const SampleFull& S, JacConst& c) {
+    for (int i = 0; i < 9; ++i) c.Ms[i] = (float)S.Ms[i];
+    for (int i = 0; i < 3; ++i) c.ia[i] = (float)S.ia[i];
+    for (int i = 0; i < 4; ++i) c.q[i] = (float)S.q[i];
+}
+SQ_HD void lsq_jac_row(const JacConst& c, const Bwd& b, float dx, float dy, float dz, float r, float* j) {
+    for (int i = 0; i < 3; ++i) j[i] = c.ia[i] * fmaf(-2.0f, b.wa[i], 0.5f * r);
+    j[3] = (float)kLn2 * b.ge[0];
+    j[4] = (float)kLn2 * b.ge[1];
+    for (int k = 0; k < 3; ++k) j[5 + k] = -2.0f * fmaf(c.Ms[k], b.gs[0], fmaf(c.Ms[3 + k], b.gs[1], c.Ms[6 + k] * b.gs[2]));
+    float u[3];                                               // dF/dM_ik = u_i d_k
+    for (int i = 0; i < 3; ++i) u[i] = 2.0f * c.ia[i] * b.gs[i];
+    const float g00 = u[0] * dx, g01 = u[0] * dy, g02 = u[0] * dz, g10 = u[1] * dx, g11 = u[1] * dy, g12 = u[1] * dz,
+                g20 = u[2] * dx, g21 = u[2] * dy, g22 = u[2] * dz;
+    const float x = c.q[0], y = c.q[1], z = c.q[2], w = c.q[3];
+    j[8]  = 2.0f * (y * (g01 + g10) + z * (g02 + g20) + w * (g12 - g21) - 2.0f * x * (g11 + g22));
+    j[9]  = 2.0f * (x * (g01 + g10) + z * (g12 + g21) + w * (g20 - g02) - 2.0f * y * (g00 + g22));
+    j[10] = 2.0f * (x * (g02 + g20) + y * (g12 + g21) + w * (g01 - g10) - 2.0f * z * (g00 + g11));
+    j[11] = 2.0f * (z * (g01 - g10) + y * (g20 - g02) + x * (g12 - g21));
+}
+
 // ---------------------------------------------------------------- LeastSquares: one point
 // classes.py:322-355: (sqrt(a1 a2 a3) (F - 1))^2 at a back-projected depth pixel (x, y, z).  Returns the squared
 // term without the a1 a2 a3 factor; accumulates d/dF-weighted terms.  The a-gradient of the prefactor is added in
 // finalize from the returned sum.
-template <bool BWD>
-SQ_HD float lsq_point(const Sample& S, float px, float py, float pz, Acc& acc) {
+// GN (normal equations): also adds the point's Jacobian row (lsq_jac_row) into jtj[kJtJN]; a point with F >= 1e18 adds
+// nothing there, as it adds nothing to the gradient.
+template <bool BWD, bool GN = false>
+SQ_HD float lsq_point(const Sample& S, float px, float py, float pz, Acc& acc, const JacConst* jc = nullptr,
+                      float* jtj = nullptr) {
     const double dx = (double)px - S.t[0], dy = (double)py - S.t[1], dz = (double)pz - S.t[2];
     float s[3];
     for (int i = 0; i < 3; ++i) s[i] = (float)(S.Ms[3 * i] * dx + S.Ms[3 * i + 1] * dy + S.Ms[3 * i + 2] * dz);
@@ -1600,6 +1636,17 @@ SQ_HD float lsq_point(const Sample& S, float px, float py, float pz, Acc& acc) {
         }
         acc.ge[0] += b.ge[0];
         acc.ge[1] += b.ge[1];
+        if (GN) {
+            Bwd bj;
+            point_backward(fa, ok ? 1.f : 0.f, bj);
+            float j[12];
+            lsq_jac_row(*jc, bj, fdx, fdy, fdz, ok ? r : 0.f, j);
+            int e = 0;
+#pragma unroll
+            for (int k = 0; k < 12; ++k)
+#pragma unroll
+                for (int l = k; l < 12; ++l, ++e) jtj[e] = fmaf(j[k], j[l], jtj[e]);
+        }
     }
     return r * r;
 }

@@ -601,6 +601,27 @@ __device__ __forceinline__ void block_reduce_store(const Acc& a, float (*red)[kA
     }
 }
 
+// LeastSquares normal-equations mode: a partial row is the kRow row above, then the kJtJN sums of J^T J, then two floats of
+// padding (rows stay 16-byte aligned)
+constexpr int kRowGN = kRow + kJtJN + 2;
+
+// per-thread J^T J sums -> row[kRow ...] of the block's partial row (after block_reduce_store, with its own tile)
+__device__ __forceinline__ void block_reduce_store_jtj(const float* v, float (*red)[kJtJN], float* row) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int i = 0; i < kJtJN; ++i) {
+        const float s = warp_sum(v[i]);
+        if (lane == 0) red[warp][i] = s;
+    }
+    __syncthreads();
+    if (threadIdx.x < kJtJN) {
+        float s = 0.f;
+#pragma unroll
+        for (int w = 0; w < kWarps; ++w) s += red[w][threadIdx.x];
+        row[kRow + threadIdx.x] = s;
+    }
+}
+
 __device__ __forceinline__ void load_sample(Sample* dst, const SampleFull* src) {   // whole block
     const uint32_t* s = reinterpret_cast<const uint32_t*>(src);
     uint32_t* d = reinterpret_cast<uint32_t*>(dst);
@@ -1381,16 +1402,33 @@ __global__ void iou_export_kernel(const unsigned long long* counts, int batch, l
 // ------------------------------------------------------------------------------------------------ LeastSquares
 constexpr int kLsqPix = 4;               // pixels per thread of the point-list kernel
 
-template <bool BWD>
+// GN (normal-equations mode, BWD only): every point also adds its Jacobian row to the thread's kJtJN J^T J sums, which the
+// block reduces into columns kRow ... of its kRowGN-wide partial row.  The fp32 Jacobian constants sit in shared memory,
+// written by thread 0 before the block's first barrier.
+struct LsqGN { const JacConst* jc; float (*red)[kJtJN]; };
+__device__ __forceinline__ LsqGN lsq_gn_setup(const SampleFull* sample, float* jt) {
+    __shared__ JacConst jc;
+    __shared__ float red[kWarps][kJtJN];
+    if (threadIdx.x == 0) jac_const(*sample, jc);
+#pragma unroll
+    for (int i = 0; i < kJtJN; ++i) jt[i] = 0.f;
+    return LsqGN{&jc, red};
+}
+
+template <bool BWD, bool GN = false>
 __global__ void __launch_bounds__(kThreads)
 lsq_kernel(const SampleFull* __restrict__ samples, int R, int items_per_sample,
            const float* __restrict__ target, long long tstride, const int* __restrict__ row_off,
            const int* __restrict__ col_off, float* __restrict__ partials) {
+    static_assert(BWD || !GN, "the normal equations need the backward");
     __shared__ Sample S;
     __shared__ float red[kWarps][kAccN];
     const int item = blockIdx.x;
     const int b = item / items_per_sample, chunk = item - b * items_per_sample;
     load_sample(&S, samples + b);
+    float jt[GN ? kJtJN : 1];
+    LsqGN gn{nullptr, nullptr};
+    if constexpr (GN) gn = lsq_gn_setup(samples + b, jt);
     __syncthreads();
     Acc acc;
     acc_zero(acc);
@@ -1412,10 +1450,12 @@ lsq_kernel(const SampleFull* __restrict__ samples, int R, int items_per_sample,
         if (v[k] > 0.f) {                                  // classes.py:363-368 (fp32 arithmetic, like the reference)
             const int row = pixs[k] / R, col = pixs[k] - row * R;
             const float px = (float)col / (float)R, py = 1.0f - (float)row / (float)R;
-            acc.loss += lsq_point<BWD>(S, px, py, v[k], acc);
+            acc.loss += lsq_point<BWD, GN>(S, px, py, v[k], acc, gn.jc, jt);
         }
     }
-    block_reduce_store(acc, red, partials + (size_t)item * kRow);
+    float* row = partials + (size_t)item * (GN ? kRowGN : kRow);
+    block_reduce_store(acc, red, row);
+    if constexpr (GN) block_reduce_store_jtj(jt, gn.red, row);
 }
 
 // LeastSquares.energy_function on an explicit, compacted point list (classes.py:318-356): structure of arrays x[], y[],
@@ -1424,15 +1464,19 @@ lsq_kernel(const SampleFull* __restrict__ samples, int R, int items_per_sample,
 // points of each coordinate row with one 16-byte load.  The chunk grid is aligned to multiples of four points of the
 // WHOLE buffer (rows are 16-byte aligned and padded to a multiple of four), points outside the sample's range are masked.
 // 12 bytes per point from HBM, read once.
-template <bool BWD>
+template <bool BWD, bool GN = false>
 __global__ void __launch_bounds__(kThreads)
 lsq_points_kernel(const SampleFull* __restrict__ samples, int chunks_per_sample, const float* __restrict__ points,
                   long long stride, const long long* __restrict__ offsets, float* __restrict__ partials) {
+    static_assert(BWD || !GN, "the normal equations need the backward");
     __shared__ Sample S;
     __shared__ float red[kWarps][kAccN];
     const int item = blockIdx.x;
     const int b = item / chunks_per_sample, chunk = item - b * chunks_per_sample;
     load_sample(&S, samples + b);
+    float jt[GN ? kJtJN : 1];
+    LsqGN gn{nullptr, nullptr};
+    if constexpr (GN) gn = lsq_gn_setup(samples + b, jt);
     __syncthreads();
     Acc acc;
     acc_zero(acc);
@@ -1445,14 +1489,17 @@ lsq_points_kernel(const SampleFull* __restrict__ samples, int chunks_per_sample,
         const float xs[4] = {x4.x, x4.y, x4.z, x4.w}, ys[4] = {y4.x, y4.y, y4.z, y4.w}, zs[4] = {z4.x, z4.y, z4.z, z4.w};
 #pragma unroll
         for (int k = 0; k < 4; ++k)
-            if (base + k >= lo && base + k < hi) acc.loss += lsq_point<BWD>(S, xs[k], ys[k], zs[k], acc);
+            if (base + k >= lo && base + k < hi) acc.loss += lsq_point<BWD, GN>(S, xs[k], ys[k], zs[k], acc, gn.jc, jt);
     }
-    block_reduce_store(acc, red, partials + (size_t)item * kRow);
+    float* row = partials + (size_t)item * (GN ? kRowGN : kRow);
+    block_reduce_store(acc, red, row);
+    if constexpr (GN) block_reduce_store_jtj(jt, gn.red, row);
 }
 
 // ------------------------------------------------------------------------------------------------ finalize
-enum { FIN_IMPLICIT = 0, FIN_EXPLICIT = 1, FIN_LSQ = 2, FIN_OCC_VJP = 3 };     // FIN_OCC_VJP: z moment about plane_of_t()
-                                                                               // (sq_occupancy_vjp and sq_voxel_loss)
+enum { FIN_IMPLICIT = 0, FIN_EXPLICIT = 1, FIN_LSQ = 2, FIN_OCC_VJP = 3, FIN_LSQ_GN = 4 };     // FIN_OCC_VJP: z moment about
+                                                         // plane_of_t() (sq_occupancy_vjp and sq_voxel_loss); FIN_LSQ_GN:
+                                                         // FIN_LSQ on kRowGN-wide rows, plus J^T J into `jtj`
 
 // One block of kFinThreads per sample: every thread sums the partial rows r = t, t + kFinThreads, ... in fp64 (all loads
 // independent: one L2 round trip), a fixed-order tree (shuffles inside a warp, then the warps in index order) gives the
@@ -1469,7 +1516,10 @@ finalize_kernel(const SampleFull* __restrict__ samples, Grid g, int batch, int i
                 const float* __restrict__ partials, double loss_norm, double grad_scale,
                 int dtype, void* __restrict__ grad, double* __restrict__ per_sample,
                 double* __restrict__ per_sample_user, double* __restrict__ loss_out, unsigned int* ticket,
-                const double* __restrict__ loss_offset, const unsigned char* __restrict__ item_class) {
+                const double* __restrict__ loss_offset, const unsigned char* __restrict__ item_class,
+                double* __restrict__ jtj) {
+    constexpr bool kLsq = KIND == FIN_LSQ || KIND == FIN_LSQ_GN;
+    constexpr int kRS = KIND == FIN_LSQ_GN ? kRowGN : kRow;       // floats per partial row
     const int b = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
     __shared__ SampleFull S;
     __shared__ double wpart[kFinThreads / 32][kAccN];
@@ -1482,11 +1532,11 @@ finalize_kernel(const SampleFull* __restrict__ samples, Grid g, int batch, int i
         double s[kAccN];
 #pragma unroll
         for (int i = 0; i < kAccN; ++i) s[i] = 0.0;
-        const float* base = partials + (size_t)b * items_per_sample * kRow;
+        const float* base = partials + (size_t)b * items_per_sample * kRS;
         for (int j = t; j < items_per_sample; j += kFinThreads) {
             // items the plan kernel proved empty were never processed: they have no row (and contribute nothing)
             if (item_class && item_class[(size_t)b * items_per_sample + j] == kClasses - 1) continue;
-            const float4* p = reinterpret_cast<const float4*>(base + (size_t)j * kRow);      // rows are 80 bytes: 16-aligned
+            const float4* p = reinterpret_cast<const float4*>(base + (size_t)j * kRS);       // rows are 80 (400) bytes: 16-aligned
             float v[kRow];
 #pragma unroll
             for (int i = 0; i < kRow / 4; ++i) { const float4 q = __ldcg(p + i); v[4 * i] = q.x; v[4 * i + 1] = q.y; v[4 * i + 2] = q.z; v[4 * i + 3] = q.w; }
@@ -1509,7 +1559,7 @@ finalize_kernel(const SampleFull* __restrict__ samples, Grid g, int batch, int i
         acc[t] = v;
     }
     __syncthreads();
-    const double vol = KIND == FIN_LSQ ? S.a[0] * S.a[1] * S.a[2] : 1.0;
+    const double vol = kLsq ? S.a[0] * S.a[1] * S.a[2] : 1.0;
     if (warp == 1) {
         // Loss path, next to the gradient path of warp 0: per-sample loss, then the batch mean by the last block to
         // arrive, in index order.
@@ -1532,13 +1582,29 @@ finalize_kernel(const SampleFull* __restrict__ samples, Grid g, int batch, int i
         }
     } else if (t == 0 && grad) {
         double gr[12];
-        finalize_sample(S, g, acc, grad_scale * vol, KIND != FIN_LSQ, gr, KIND == FIN_OCC_VJP ? (double)plane_of_t(S, g) : 0.0);
-        if (KIND == FIN_LSQ)
+        finalize_sample(S, g, acc, grad_scale * vol, !kLsq, gr, KIND == FIN_OCC_VJP ? (double)plane_of_t(S, g) : 0.0);
+        if (kLsq)
             for (int i = 0; i < 3; ++i) gr[i] += S.mask[i] * (vol * S.ia[i]) * acc[17] * (0.5 * grad_scale);   // d (a1 a2 a3) / d a_i
         if (S.heads) heads_backward(S.hp, S.hrn, S.q, gr);
         for (int i = 0; i < 12; ++i) {
             if (dtype == SQ_F64) static_cast<double*>(grad)[12 * (size_t)b + i] = gr[i];
             else static_cast<float*>(grad)[12 * (size_t)b + i] = (float)gr[i];
+        }
+    }
+    if constexpr (KIND == FIN_LSQ_GN) {
+        // J^T J = a1 a2 a3 sum_pts j j^T: thread t < kJtJN sums upper-triangle entry t (row k, column l) over the partial rows
+        // in index order and writes it to both halves; a clamped-out parameter's row and column are exactly zero
+        if (t < kJtJN) {
+            int k = 0, e = t;
+            while (e >= 12 - k) { e -= 12 - k; ++k; }
+            const int l = k + e;
+            const float* col = partials + (size_t)b * items_per_sample * kRowGN + kRow + t;
+            double s = 0.0;
+            for (int j = 0; j < items_per_sample; ++j) s += (double)__ldcg(col + (size_t)j * kRowGN);
+            const bool live = (k >= 8 || S.mask[k] != 0.f) && (l >= 8 || S.mask[l] != 0.f);
+            const double v = live ? vol * s : 0.0;
+            jtj[144 * (size_t)b + 12 * k + l] = v;
+            jtj[144 * (size_t)b + 12 * l + k] = v;
         }
     }
 }
@@ -1836,7 +1902,8 @@ static int implicit_loss_impl(const void* pred, int pred_dtype, int batch, int n
         SQ_TRY(launch_dependent(finalize_kernel<FIN_IMPLICIT>, batch, kFinThreads, 0, st, pdl,
                                 s.pred, g, batch, L.rows_per_sample, s.partials, 1.0 / nn,
                                 -(double)sharpness * (double)tau / (nn * n * (double)batch), pred_dtype, grad_pred, s.per_sample,
-                                per_sample, loss_out, &s.ctl->ticket, s.tv_sum, queue ? s.item_class : nullptr));
+                                per_sample, loss_out, &s.ctl->ticket, s.tv_sum, queue ? s.item_class : nullptr,
+                                static_cast<double*>(nullptr)));
         SQ_TRY(cudaGetLastError());
     }
 #endif
@@ -1899,7 +1966,8 @@ int sq_depth_projection_vjp(const void* pred, int pred_dtype, int batch, int n, 
     SQ_TRY(launch_dependent(finalize_kernel<FIN_IMPLICIT>, batch, kFinThreads, 0, st, pdl,
                             s.pred, g, batch, L.rows_per_sample, s.partials, 0.0, -(double)sharpness * (double)tau / (double)n,
                             pred_dtype, grad_pred, s.per_sample, static_cast<double*>(nullptr), static_cast<double*>(nullptr),
-                            &s.ctl->ticket, static_cast<const double*>(nullptr), queue ? s.item_class : nullptr));
+                            &s.ctl->ticket, static_cast<const double*>(nullptr), queue ? s.item_class : nullptr,
+                            static_cast<double*>(nullptr)));
     SQ_TRY(cudaGetLastError());
     return 0;
 }
@@ -1930,7 +1998,7 @@ int sq_explicit_loss(const void* true_params, const void* pred, int params_dtype
     finalize_kernel<FIN_EXPLICIT><<<batch, kFinThreads, 0, st>>>(
         s.pred, g, batch, L.rows_per_sample, s.partials, (double)mult / n3,
         2.0 * (double)sharpness * (double)mult / (n3 * (double)batch), params_dtype, grad_pred, s.per_sample,
-        per_sample, loss_out, &s.ctl->ticket, nullptr, queue ? s.item_class : nullptr);
+        per_sample, loss_out, &s.ctl->ticket, nullptr, queue ? s.item_class : nullptr, nullptr);
     SQ_TRY(cudaGetLastError());
     return 0;
 }
@@ -1962,7 +2030,7 @@ int sq_occupancy_vjp(const void* params, int params_dtype, int batch, int n, dou
     SQ_TRY(cudaGetLastError());
     finalize_kernel<FIN_OCC_VJP><<<batch, kFinThreads, 0, st>>>(
         s.pred, g, batch, L.rows_per_sample, s.partials, 0.0, -(double)sharpness, params_dtype, grad_params, s.per_sample,
-        nullptr, nullptr, &s.ctl->ticket, nullptr, queue ? s.item_class : nullptr);
+        nullptr, nullptr, &s.ctl->ticket, nullptr, queue ? s.item_class : nullptr, nullptr);
     SQ_TRY(cudaGetLastError());
     return 0;
 }
@@ -2007,7 +2075,7 @@ int sq_voxel_loss(const void* voxels, int voxel_dtype, float voxel_scale,
     finalize_kernel<FIN_OCC_VJP><<<batch, kFinThreads, 0, st>>>(
         s.pred, g, batch, L.rows_per_sample, s.partials, (double)mult / n3,
         2.0 * (double)sharpness * (double)mult / (n3 * (double)batch), params_dtype, grad_pred, s.per_sample,
-        per_sample, loss_out, &s.ctl->ticket, nullptr, nullptr);
+        per_sample, loss_out, &s.ctl->ticket, nullptr, nullptr, nullptr);
     SQ_TRY(cudaGetLastError());
     return 0;
 }
@@ -2055,7 +2123,7 @@ int sq_least_squares(const void* pred, int pred_dtype, int batch, int render_siz
     SQ_TRY(cudaGetLastError());
     finalize_kernel<FIN_LSQ><<<batch, kFinThreads, 0, st>>>(s.pred, g, batch, ips, s.partials, 1.0, 2.0 / (double)batch,
                                                    pred_dtype, grad_pred, s.per_sample, per_sample, loss_out, &s.ctl->ticket,
-                                                   nullptr, nullptr);
+                                                   nullptr, nullptr, nullptr);
     SQ_TRY(cudaGetLastError());
     return 0;
 }
@@ -2081,7 +2149,8 @@ int sq_least_squares_points(const void* pred, int pred_dtype, int batch, const f
     SQ_TRY(cudaGetLastError());
     // per-sample energies: the gradient is d per_sample[b] / d pred[b] (no 1 / batch)
     finalize_kernel<FIN_LSQ><<<batch, kFinThreads, 0, st>>>(s.pred, g, batch, chunks, s.partials, 1.0, 2.0, pred_dtype, grad_pred,
-                                                   s.per_sample, per_sample, loss_out, &s.ctl->ticket, nullptr, nullptr);
+                                                   s.per_sample, per_sample, loss_out, &s.ctl->ticket, nullptr, nullptr,
+                                                   nullptr);
     SQ_TRY(cudaGetLastError());
     return 0;
 }
@@ -2093,6 +2162,89 @@ size_t sq_points_scratch_bytes(int batch, long long max_points) {
     int n = 1;
     while ((long long)n * n < (long long)chunks * kThreads) ++n;
     return scratch_layout(batch, n, nullptr, nullptr);
+}
+
+// ---- LeastSquares normal equations: per-sample energy, gradient and J^T J (sq_least_squares_normal / _points_normal)
+// Scratch: the control block, one SampleFull per sample, kRowGN-wide partial rows (`chunks` per sample), the energies.
+static int lsq_point_chunks(long long max_points) {       // blocks of kThreads * 4 points per sample (sq_least_squares_points)
+    const long long chunks64 = (max_points + 3 + kThreads * 4 - 1) / (kThreads * 4);
+    return chunks64 > 0 ? (int)chunks64 : 1;
+}
+
+static size_t normal_layout(int batch, int chunks, char* base, Scratch* s) {
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
+    const size_t o_ctl = take(sizeof(Control));
+    const size_t o_pred = take(sizeof(SampleFull) * (size_t)batch);
+    const size_t o_part = take(sizeof(float) * kRowGN * (size_t)chunks * (size_t)batch);
+    const size_t o_ps = take(sizeof(double) * (size_t)batch);
+    if (s) {
+        *s = Scratch{};
+        s->ctl = reinterpret_cast<Control*>(base + o_ctl);
+        s->pred = reinterpret_cast<SampleFull*>(base + o_pred);
+        s->partials = reinterpret_cast<float*>(base + o_part);
+        s->per_sample = reinterpret_cast<double*>(base + o_ps);
+    }
+    return off;
+}
+
+size_t sq_normal_scratch_bytes(int batch, long long max_points) {
+    if (batch <= 0 || max_points < 0) return 0;
+    return normal_layout(batch, lsq_point_chunks(max_points), nullptr, nullptr);
+}
+
+static int normal_scratch(int batch, int chunks, void* scratch, size_t bytes, Scratch* s) {
+    if (batch <= 0 || !scratch || bytes < normal_layout(batch, chunks, nullptr, nullptr)) return (int)cudaErrorInvalidValue;
+    normal_layout(batch, chunks, static_cast<char*>(scratch), s);
+    return 0;
+}
+
+int sq_least_squares_normal(const void* pred, int pred_dtype, int batch, int render_size, const float* target,
+                            long long target_stride_b, const int* row_off, const int* col_off,
+                            double* per_sample, void* grad_pred, double* jtj,
+                            void* scratch, size_t scratch_bytes, sq_stream_t stream) {
+    if (!pred || !target || !row_off || !col_off || !per_sample || !grad_pred || !jtj || render_size <= 0 ||
+        render_size > 46340)
+        return (int)cudaErrorInvalidValue;
+    const int R = render_size;
+    const int ips = (R * R + kThreads * kLsqPix - 1) / (kThreads * kLsqPix);
+    Scratch s;
+    int rc = normal_scratch(batch, ips, scratch, scratch_bytes, &s);
+    if (rc) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const Grid g = make_grid(2, 1.0, 0.0);     // the point list carries its own coordinates; the grid is unused
+    rc = launch_prep(pred, pred_dtype, batch, true, g, s.pred, s.ctl, st);
+    if (rc) return rc;
+    lsq_kernel<true, true><<<batch * ips, kThreads, 0, st>>>(s.pred, R, ips, target, target_stride_b, row_off, col_off, s.partials);
+    SQ_TRY(cudaGetLastError());
+    finalize_kernel<FIN_LSQ_GN><<<batch, kFinThreads, 0, st>>>(s.pred, g, batch, ips, s.partials, 1.0, 2.0, pred_dtype, grad_pred,
+                                                      s.per_sample, per_sample, nullptr, &s.ctl->ticket, nullptr, nullptr,
+                                                      jtj);
+    SQ_TRY(cudaGetLastError());
+    return 0;
+}
+
+int sq_least_squares_points_normal(const void* pred, int pred_dtype, int batch, const float* points, long long stride,
+                                   const long long* offsets, long long max_points,
+                                   double* per_sample, void* grad_pred, double* jtj,
+                                   void* scratch, size_t scratch_bytes, sq_stream_t stream) {
+    if (!pred || !points || !offsets || max_points < 0 || stride < 0 || (stride & 3) || !per_sample || !grad_pred || !jtj)
+        return (int)cudaErrorInvalidValue;
+    const int chunks = lsq_point_chunks(max_points);
+    Scratch s;
+    int rc = normal_scratch(batch, chunks, scratch, scratch_bytes, &s);
+    if (rc) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const Grid g = make_grid(2, 1.0, 0.0);
+    rc = launch_prep(pred, pred_dtype, batch, true, g, s.pred, s.ctl, st);
+    if (rc) return rc;
+    lsq_points_kernel<true, true><<<batch * chunks, kThreads, 0, st>>>(s.pred, chunks, points, stride, offsets, s.partials);
+    SQ_TRY(cudaGetLastError());
+    finalize_kernel<FIN_LSQ_GN><<<batch, kFinThreads, 0, st>>>(s.pred, g, batch, chunks, s.partials, 1.0, 2.0, pred_dtype,
+                                                      grad_pred, s.per_sample, per_sample, nullptr, &s.ctl->ticket, nullptr,
+                                                      nullptr, jtj);
+    SQ_TRY(cudaGetLastError());
+    return 0;
 }
 
 int sq_field(const void* params, int params_dtype, int batch, int n, double step, double z0, int mode,

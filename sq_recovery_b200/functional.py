@@ -300,6 +300,66 @@ def lsq_energy(batch_points, params: torch.Tensor) -> torch.Tensor:
     return LsqEnergyFn.apply(params, packed, offsets, max_points, torch.is_grad_enabled())
 
 
+def _normal_outputs(p: torch.Tensor):
+    B = p.shape[0]
+    return (torch.empty(B, dtype=torch.float64, device=p.device), torch.empty_like(p),
+            torch.empty((B, 12, 12), dtype=torch.float64, device=p.device))
+
+
+def lsq_normal_equations(true: torch.Tensor, pred: torch.Tensor, render_size: int):
+    """LeastSquares normal equations on depth images (sq_least_squares_normal): per sample the energy E_b (B,) fp64,
+    dE_b / dpred_b (B, 12) in pred's dtype and J_b^T J_b (B, 12, 12) fp64.  No autograd history; pred is read detached."""
+    _require_cuda(pred, "pred"); _require_cuda(true, "true")
+    dev = pred.device
+    if true.device != dev:
+        raise ValueError(f"true ({true.device}) must be on pred's device ({dev})")
+    img = _image(true)
+    p, tag = _params(pred)
+    B = p.shape[0]
+    if img.shape[0] != B:
+        raise ValueError("true and pred disagree on the batch size")
+    row_off, col_off = nearest_offsets(img.shape[2], img.shape[3], render_size, dev)
+    energy, grad, jtj = _normal_outputs(p)
+    L = _lib.lib()
+    scratch = _get_scratch(dev, B, 0, need=L.sq_normal_scratch_bytes(B, render_size * render_size))
+    with _on_device(dev):
+        rc = L.sq_least_squares_normal(_ptr(p), tag, B, render_size, _ptr(img), img.shape[2] * img.shape[3], _ptr(row_off),
+                                       _ptr(col_off), _ptr(energy), _ptr(grad), _ptr(jtj), _ptr(scratch), scratch.numel(),
+                                       _stream(dev))
+    _lib.check(rc, "sq_least_squares_normal")
+    return energy, grad.to(pred.dtype), jtj
+
+
+def lsq_points_normal_equations(batch_points, params: torch.Tensor):
+    """LeastSquares normal equations on point lists (sq_least_squares_points_normal): the outputs of
+    lsq_normal_equations for the (3, m_i) lists of energy_function."""
+    _require_cuda(params, "params")
+    if params.dim() != 2 or len(batch_points) != params.shape[0]:
+        raise ValueError("one point list per parameter row is required")
+    dev = params.device
+    for pts in batch_points:
+        if isinstance(pts, torch.Tensor) and pts.device != dev:
+            raise ValueError(f"point lists ({pts.device}) must be on params' device ({dev})")
+    return lsq_points_normal_packed(params, *pack_points(batch_points, dev))
+
+
+def lsq_points_normal_packed(params: torch.Tensor, packed: torch.Tensor, offsets: torch.Tensor, max_points: int):
+    """lsq_points_normal_equations on lists already packed by pack_points: no host-to-device copy, so the call can be
+    captured into a CUDA graph."""
+    p, tag = _params(params)
+    B = p.shape[0]
+    dev = params.device
+    energy, grad, jtj = _normal_outputs(p)
+    L = _lib.lib()
+    scratch = _get_scratch(dev, B, 0, need=L.sq_normal_scratch_bytes(B, max_points))
+    with _on_device(dev):
+        rc = L.sq_least_squares_points_normal(_ptr(p), tag, B, _ptr(packed), packed.shape[1], _ptr(offsets), max_points,
+                                              _ptr(energy), _ptr(grad), _ptr(jtj), _ptr(scratch), scratch.numel(),
+                                              _stream(dev))
+    _lib.check(rc, "sq_least_squares_points_normal")
+    return energy, grad.to(params.dtype), jtj
+
+
 def iou_counts(true: torch.Tensor, pred: torch.Tensor, n: int, step: float, z0: float = 0.0):
     """(intersection[B], union[B]) int64 voxel counts of F<=1 (torch/classes.py:433-438).  Forward only."""
     _require_cuda(pred, "pred"); _require_cuda(true, "true")

@@ -15,8 +15,9 @@ return is scaled back by the batch size.  Pairs are sharded over the ranks; no c
 --loss voxels-fused is the same objective through ExplicitLoss.voxel_loss: the target is that grid as bool (read as bytes),
 loss and gradient are one fused walk, and no occupancy grid is held in memory.
 --loss lsq descends through LeastSquares(R) on the same 256^2 depth renders --loss implicit uses.  --method lm (with --loss
-lsq only) replaces the descent by a batched Levenberg-Marquardt fit on LeastSquares.normal_equations: `--steps` iterations,
-each one solve per sample and one normal-equations call at the trial point (levenberg_marquardt below).
+lsq or implicit) replaces the descent by a batched Levenberg-Marquardt fit on LeastSquares.normal_equations, or on
+ImplicitLoss.render_normal_equations (the squared depth residual of the render against the resized image): `--steps`
+iterations, each one solve per sample and one normal-equations call at the trial point (levenberg_marquardt below).
 Prints one JSON line on rank 0: steps/s, loss evaluations (grid points) per second, IoU(128) before / after.
 """
 import argparse
@@ -116,8 +117,8 @@ def main():
     ap.add_argument("--loss", default="explicit", choices=["explicit", "implicit", "voxels", "voxels-fused", "lsq"])
     ap.add_argument("--method", default="gd", choices=["gd", "lm"])
     args = ap.parse_args()
-    if args.method == "lm" and args.loss != "lsq":
-        ap.error("--method lm needs --loss lsq (the only sum-of-squares loss)")
+    if args.method == "lm" and args.loss not in ("lsq", "implicit"):
+        ap.error("--method lm needs --loss lsq or --loss implicit (the losses with normal equations)")
     import sq_recovery_b200 as S
     from sq_recovery_b200 import distributed as D
     from sq_recovery_b200 import inputs as O          # seeded randsq / randquat workloads
@@ -150,8 +151,10 @@ def main():
     iou = S.IoUAccuracy(128, dev)
     i0, u0 = iou.counts(true, pred)
     if args.method == "lm":
+        normal = crit.normal_equations if args.loss == "lsq" else crit.render_normal_equations
+
         def fit(p, steps, record=None):
-            levenberg_marquardt(crit.normal_equations, target, p, steps, record=record)
+            levenberg_marquardt(normal, target, p, steps, record=record)
     else:
         def fit(p, steps, record=None):
             descend(crit, target, p, steps, record=record)
@@ -165,7 +168,7 @@ def main():
     fit(pred, args.steps, rec)
     e1.record()
     torch.cuda.synchronize()
-    if args.method == "lm":                                 # batch-mean energy, the scale of LeastSquares' loss
+    if args.method == "lm":                                 # batch-mean energy (LeastSquares' loss; implicit: sum of r^2)
         rec = [E.mean() for E, _ in rec]
     ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     i1, u1 = iou.counts(true, pred)

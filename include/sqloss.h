@@ -90,6 +90,18 @@ int sq_depth_projection_vjp(const void* pred, int pred_dtype, int batch, int n, 
                             float tau, float sharpness, const float* grad_depth, void* grad_pred,
                             void* scratch, size_t scratch_bytes, sq_stream_t stream);
 
+/* Jacobian of ImplicitLoss.depth_projection (torch/classes.py:232-282), one row per pixel:
+ *   jac        [batch,n,n,12] fp32, image orientation: jac[b,r,c,j] = d depth[b,r,c] / d pred[b,j]
+ *              (clamp masks as in the loss; quaternion not normalised).  fp32 for fp32 and fp64 pred alike: each entry
+ *              is an fp32 sum, and fp64 storage would double the call's largest buffer (48 bytes per pixel).
+ *   depth_out  [batch,n,n] fp32 render of the same walk (may be NULL)
+ * Weight cut of one sample (as sq_depth_projection_vjp): row (b,r,c) is that call's result for a one-hot grad_depth on
+ * pixel (b,r,c).  Scratch: sq_scratch_bytes(batch, n), usual control-block contract.  Asynchronous, self-contained,
+ * capturable; its column kernel is timed by sq_profile_events.  NULL pred or jac: cudaErrorInvalidValue. */
+int sq_depth_projection_jacobian(const void* pred, int pred_dtype, int batch, int n, double step, double z0,
+                                 float tau, float sharpness, float* depth_out, float* jac,
+                                 void* scratch, size_t scratch_bytes, sq_stream_t stream);
+
 /* ExplicitLoss.__call__ (torch/classes.py:138-201): mean_b( mult * mean_pts (o_true - o_pred)^2 ),
  * o = sigmoid(sharpness (1 - F)); the reference uses sharpness 5, mult 100 (:187, :198).
  *   grad_pred   [batch,12] d loss / d pred (params_dtype)              (NULL = forward only)

@@ -145,6 +145,25 @@ class ImplicitLoss(_GridLoss):
             return Fn.DepthProjectionFn.apply(p, *args)
         return Fn.depth_projection(p, *args)
 
+    def render_jacobian(self, p):
+        """``(depth (B, R, R) fp32, jac (B, R, R, 12) fp32)``: the render and its Jacobian row per pixel,
+        jac[b, r, c, j] = d depth[b, r, c] / d p[b, j] in image orientation (clamp masks as in the loss, quaternion not
+        normalised), from one CUDA walk.  Row (b, r, c) is the VJP of ``render`` for a one-hot upstream on that pixel.
+        Plain tensors; ``p`` is read detached in any grad mode.  jac is fp32 for fp32 and fp64 ``p`` alike and takes
+        48 R^2 bytes per sample: 50 MB at B = 256, R = 64, and 3 MB per sample at R = 256."""
+        return Fn.depth_jacobian(p, self._n, self._step, self._z0, float(self.tau), float(self.sigmoid_sharpness))
+
+    def render_normal_equations(self, true, pred, weight=None):
+        """Gauss-Newton normal equations of the weighted squared depth residual r = render(pred) - t per sample, where
+        t is the (B, 1, H, W) image ``true`` sampled nearest to R x R exactly as ``self(true, pred)`` samples it:
+        ``(E (B,) fp64, g (B, 12) in pred's dtype, H (B, 12, 12) fp64)`` with E_b = sum w r^2, g_b = 2 J_b^T W r_b and
+        H_b = J_b^T W J_b, J from ``render_jacobian``.  This is the L2 image residual, not the MAE the loss call returns;
+        ``weight`` (B, R, R), image orientation, non-negative (not checked), turns it into IRLS on that MAE
+        (w = 1 / max(|r|, eps)) or masks pixels.  No 1 / B factor, no autograd history.  The signature is that of
+        ``LeastSquares.normal_equations``, so harness/optimize.py's levenberg_marquardt takes either."""
+        return Fn.render_normal_equations(true, pred, weight, self._n, self._step, self._z0, float(self.tau),
+                                          float(self.sigmoid_sharpness))
+
     def __call__(self, true, pred):
         return Fn.ImplicitLossFn.apply(true, pred, self._n, self._step, self._z0, float(self.tau),
                                        float(self.sigmoid_sharpness), False, torch.is_grad_enabled())

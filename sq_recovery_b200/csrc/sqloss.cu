@@ -782,14 +782,28 @@ __device__ unsigned long long g_phase[8];
 constexpr size_t kImplicitBwdSmemPerWarp = (size_t)kBwdPool * 4 * sizeof(float) + 11 * 32 * sizeof(float);
 static_assert(kImplicitBwdSmemPerWarp % 32 == 0, "per-warp regions stay 32-byte aligned (BwdQueue::where carries the lane in its low bits)");
 
+// Jacobian mode of the fwd+bwd kernel (sq_depth_projection_jacobian): the rows d depth[b, row, col] / d pred[b] and
+// finalize's scale d depth / d theta = -k tau / n.  It is passed as one extra kernel argument, so that the kernels without
+// it keep their parameter list.
+struct JacOut { float* jac; double scale; };
+__device__ __forceinline__ JacOut jac_out() { return JacOut{nullptr, 0.0}; }
+__device__ __forceinline__ JacOut jac_out(JacOut j) { return j; }
+// per warp, after the pool and the column values: one deal-out round's 32 backward results (Bwd gs[3], wa[3], ge[2])
+constexpr size_t kJacStageBytesPerWarp = 8 * 32 * sizeof(float);
+
 // VJP (with BWD; sq_depth_projection_vjp): `target` is the upstream gradient dL/d depth [batch, n, n] in image orientation and
 // takes the place of sign(depth - target) as the column's weight; no loss, no depth, partial-row slots 17-19 stay 0.
-template <bool BWD, int THREADS, int MINB, int CPTMAX, bool VJP = false>      // CPTMAX: upper limit of L.cpt
+// JAC (with BWD; one JacOut argument): the column weight is 1 on valid lanes, every column keeps its own sums -- each
+// deal-out round is staged in shared memory and every lane folds in, in entry order, the entries of its own column -- and
+// each valid lane writes its column's 12-entry row and its depth.  No target, no loss, no partial rows.
+template <bool BWD, int THREADS, int MINB, int CPTMAX, bool VJP = false, typename... Jac>      // CPTMAX: upper limit of L.cpt
 __global__ void __launch_bounds__(THREADS, MINB)
 implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, ImplicitParams P, int total_items,
                 Control* __restrict__ ctl, const int* __restrict__ queue, int cap,
                 const float* __restrict__ target, long long tstride, const int* __restrict__ row_off,
-                const int* __restrict__ col_off, float* __restrict__ partials, float* __restrict__ depth_out) {
+                const int* __restrict__ col_off, float* __restrict__ partials, float* __restrict__ depth_out, Jac... jac) {
+    constexpr bool JAC = sizeof...(Jac) > 0;
+    static_assert(!JAC || (BWD && !VJP && CPTMAX == 1), "the Jacobian mode is a mode of the fwd+bwd kernel");
     __shared__ Sample Ssh[THREADS / 32];
 #if SQ_TILE_ALIAS && defined(SQ_BWD_COMPACT)
     // the fwd+bwd kernel's reduction tile lives in the warp's pool arrays, which are dead by the time the item's sums
@@ -804,8 +818,11 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
                             // points (BwdQueue arrays), per-column data for them
     constexpr int kQN = kBwdPool;
     extern __shared__ __align__(32) unsigned char dyn_smem[];
-    float* const qbuf = reinterpret_cast<float*>(dyn_smem + (size_t)(threadIdx.x >> 5) * kImplicitBwdSmemPerWarp);      // [4][kQN]
+    float* const qbuf = reinterpret_cast<float*>(dyn_smem + (size_t)(threadIdx.x >> 5) *
+                                                 (kImplicitBwdSmemPerWarp + (JAC ? kJacStageBytesPerWarp : 0)));    // [4][kQN]
     float* const colinfo_w = qbuf + 4 * kQN;                                                                         // [11][32]
+#else
+    static_assert(!JAC, "the Jacobian mode needs SQ_BWD_COMPACT");
 #endif
 #if SQ_TILE_ALIAS && defined(SQ_BWD_COMPACT)
     float* const tile_w = BWD ? qbuf : tiles_static[threadIdx.x >> 5];
@@ -981,7 +998,10 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
 #pragma unroll
                     for (int q = 1; q < CPTMAX; ++q) tv = k == q ? tvs[q] : tv;
                     asm volatile("" : "+f"(tv));
-                    if (valid && VJP) {
+                    if (valid && JAC) {
+                        if (depth_out) depth_out[((size_t)b * g.n + row) * g.n + col] = depth;
+                        wsg = 1.f;
+                    } else if (valid && VJP) {
                         wsg = tv;
                     } else if (valid) {
                         if (depth_out) depth_out[((size_t)b * g.n + row) * g.n + col] = depth;
@@ -1054,6 +1074,30 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
                                 cfq = cf_; dx_ = ci[7 * 32 + l_]; dy_ = ci[8 * 32 + l_];
                             };
                             int j = lane;
+                            if (JAC) {
+                                float* const stage = colinfo_w + 11 * 32;      // [8][32]
+                                for (; j - lane < total; j += 32) {
+                                    Bwd b0; float c0, x0, y0;
+                                    dealt(j, b0, c0, x0, y0);
+#pragma unroll
+                                    for (int i = 0; i < 3; ++i) { stage[i * 32 + lane] = b0.gs[i]; stage[(3 + i) * 32 + lane] = b0.wa[i]; }
+                                    stage[6 * 32 + lane] = b0.ge[0]; stage[7 * 32 + lane] = b0.ge[1];
+                                    __syncwarp();
+                                    // the round's entries of this lane's column, in entry order (the host build's order)
+                                    const int j0 = j - lane, m = total - j0 < 32 ? total - j0 : 32;
+                                    for (int e = 0; e < m; ++e) {
+                                        const int je = j0 + e, at = je < total_r ? je : kQN - 1 - (je - total_r);
+                                        const float tagged = qwarp.cf[at];
+                                        if (entry_lane(tagged) != lane) continue;
+                                        Bwd be;
+#pragma unroll
+                                        for (int i = 0; i < 3; ++i) { be.gs[i] = stage[i * 32 + e]; be.wa[i] = stage[(3 + i) * 32 + e]; }
+                                        be.ge[0] = stage[6 * 32 + e]; be.ge[1] = stage[7 * 32 + e];
+                                        acc_add_point(acc, be, entry_cf(S, tagged), dxy[0], dxy[1]);
+                                    }
+                                    __syncwarp();
+                                }
+                            }
 #if SQ_DENSE_ILP == 2
                             for (; j - lane + 32 < total; j += 64) {
                                 Bwd b0, b1; float c0, c1, x0, x1, y0, y1;
@@ -1071,10 +1115,29 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
                             __syncwarp();
                             SQ_PH(4);
                         }
-                        acc_to_array(acc, v);
-                        v[18] = v[19] = 0.f;
-                        tile_put(tile_w, v);
-                        folded = true;
+                        if (JAC) {
+                            if (valid) {
+                                // this column's sums -> its row, as finalize_kernel maps a sample's (sums in fp64)
+                                const JacOut jo = jac_out(jac...);
+                                double accd[kAccN];
+#pragma unroll
+                                for (int i = 0; i < 3; ++i) { accd[i] = acc.gs[i]; accd[12 + i] = acc.wa[i]; }
+#pragma unroll
+                                for (int i = 0; i < 9; ++i) accd[3 + i] = acc.gm[i];
+                                accd[15] = acc.ge[0]; accd[16] = acc.ge[1]; accd[17] = 0.0;
+                                double gr[12];
+                                finalize_sample(samples[b], g, accd, jo.scale, true, gr);
+                                float4* out = reinterpret_cast<float4*>(jo.jac + (((size_t)b * g.n + row) * g.n + col) * 12);
+#pragma unroll
+                                for (int i = 0; i < 3; ++i)
+                                    out[i] = make_float4((float)gr[4 * i], (float)gr[4 * i + 1], (float)gr[4 * i + 2], (float)gr[4 * i + 3]);
+                            }
+                        } else {
+                            acc_to_array(acc, v);
+                            v[18] = v[19] = 0.f;
+                            tile_put(tile_w, v);
+                            folded = true;
+                        }
                         SQ_PH(5);
                     }
                 } else
@@ -1968,6 +2031,48 @@ int sq_depth_projection_vjp(const void* pred, int pred_dtype, int batch, int n, 
                             pred_dtype, grad_pred, s.per_sample, static_cast<double*>(nullptr), static_cast<double*>(nullptr),
                             &s.ctl->ticket, static_cast<const double*>(nullptr), queue ? s.item_class : nullptr,
                             static_cast<double*>(nullptr)));
+    SQ_TRY(cudaGetLastError());
+    return 0;
+}
+
+// The fwd+bwd pipeline in its Jacobian mode (implicit_kernel with a JacOut): plan (as the VJP's), then the column kernel,
+// which writes every walked column's row and depth itself -- no finalize.  Columns of proven-empty items and of groups
+// with no occupancy are never touched: the call clears jac and depth_out first.
+int sq_depth_projection_jacobian(const void* pred, int pred_dtype, int batch, int n, double step, double z0,
+                                 float tau, float sharpness, float* depth_out, float* jac,
+                                 void* scratch, size_t scratch_bytes, sq_stream_t stream) {
+    Scratch s;
+    int rc = check_scratch(batch, n, scratch, scratch_bytes, &s);
+    if (rc) return rc;
+    if (!pred || !jac || (pred_dtype != SQ_F32 && pred_dtype != SQ_F64)) return (int)cudaErrorInvalidValue;      // before the clears
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const Grid g = make_grid(n, step, z0);
+    const Layout L = make_layout(n, SQ_IMPB_CPT);
+    // the VJP's weight cut of one sample: row (b, row, col) is the VJP of a one-hot upstream on that pixel
+    const ImplicitParams P{sharpness * kLog2e, tau * kLog2e, implicit_cull_bound(sharpness * kLog2e), implicit_active_bits(sharpness * kLog2e, n, 1)};
+    SQ_TRY(cudaMemsetAsync(jac, 0, sizeof(float) * 12 * (size_t)batch * n * n, st));
+    if (depth_out) SQ_TRY(cudaMemsetAsync(depth_out, 0, sizeof(float) * (size_t)batch * n * n, st));
+    rc = launch_plan(pred, nullptr, pred_dtype, batch, true, g, L, P.bound, s, nullptr, s.item_class, nullptr, st, false,
+                     SQ_WALK_ESTIMATE ? 32.0f / P.tl : 0.f);
+    if (rc) return rc;
+    const int items = batch * L.rows_per_sample;
+    const int* queue = L.rows_per_sample <= kPlanMaxItems ? s.queue : nullptr;
+#ifdef SQ_PDL
+    const bool pdl = (t_ev_before == nullptr && t_ev_after == nullptr);
+#else
+    const bool pdl = false;
+#endif
+    {
+        ColumnKernelTimer timer(st);
+        const int blocks = persistent_blocks(items, SQ_IMPB_THREADS / 32, SQ_IMPB_MINB);
+        constexpr size_t dyn = (kImplicitBwdSmemPerWarp + kJacStageBytesPerWarp) * (SQ_IMPB_THREADS / 32);
+        constexpr auto kernel = implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT, false, JacOut>;
+        SQ_TRY((opt_in_dyn_smem<kernel>(dyn)));
+        SQ_TRY(launch_dependent(kernel, blocks, SQ_IMPB_THREADS, dyn, st, pdl, s.pred, g, L, P, items, s.ctl, queue,
+                                s.queue_cap, static_cast<const float*>(nullptr), 0LL, static_cast<const int*>(nullptr),
+                                static_cast<const int*>(nullptr), static_cast<float*>(nullptr), depth_out,
+                                JacOut{jac, -(double)sharpness * (double)tau / (double)n}));
+    }
     SQ_TRY(cudaGetLastError());
     return 0;
 }

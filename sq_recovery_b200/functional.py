@@ -429,6 +429,53 @@ class DepthProjectionFn(torch.autograd.Function):
         return grad.to(ctx.pred_dtype), None, None, None, None, None
 
 
+def depth_jacobian(pred: torch.Tensor, n: int, step: float, z0: float, tau: float, sharpness: float):
+    """(depth (B, n, n) fp32, jac (B, n, n, 12) fp32) from one walk (sq_depth_projection_jacobian): the render and
+    jac[b, r, c, j] = d depth[b, r, c] / d pred[b, j], image orientation.  No autograd history; pred is read detached."""
+    _require_cuda(pred, "pred")
+    p, tag = _params(pred)
+    dev = p.device
+    B = p.shape[0]
+    depth = torch.empty((B, n, n), dtype=torch.float32, device=dev)
+    jac = torch.empty((B, n, n, 12), dtype=torch.float32, device=dev)
+    scratch = _get_scratch(dev, B, n)
+    with _on_device(dev):
+        rc = _lib.lib().sq_depth_projection_jacobian(_ptr(p), tag, B, n, step, z0, tau, sharpness, _ptr(depth), _ptr(jac),
+                                                     _ptr(scratch), scratch.numel(), _stream(dev))
+    _lib.check(rc, "sq_depth_projection_jacobian")
+    return depth, jac
+
+
+def render_normal_equations(true: torch.Tensor, pred: torch.Tensor, weight: Optional[torch.Tensor], n: int, step: float,
+                            z0: float, tau: float, sharpness: float):
+    """Normal equations of the weighted squared depth residual r = depth - t, t = `true` sampled nearest to n x n as
+    ImplicitLossFn samples it: (E (B,) fp64, g (B, 12) in pred's dtype, H (B, 12, 12) fp64) with E_b = sum w r^2,
+    g_b = 2 J_b^T W r_b, H_b = J_b^T W J_b.  J from one depth_jacobian call; both products from one batched fp64 matmul."""
+    _require_cuda(pred, "pred"); _require_cuda(true, "true")
+    dev = pred.device
+    if true.device != dev:
+        raise ValueError(f"true ({true.device}) must be on pred's device ({dev})")
+    img = _image(true)
+    B = _params(pred)[0].shape[0]
+    if img.shape[0] != B:
+        raise ValueError("true and pred disagree on the batch size")
+    if weight is not None:
+        if tuple(weight.shape) != (B, n, n):
+            raise ValueError(f"expected a weight of shape {(B, n, n)}, got {tuple(weight.shape)}")
+        if weight.device != dev:
+            raise ValueError(f"weight ({weight.device}) must be on pred's device ({dev})")
+    depth, jac = depth_jacobian(pred, n, step, z0, tau, sharpness)
+    row_off, col_off = nearest_offsets(img.shape[2], img.shape[3], n, dev)
+    t = img.view(B, -1)[:, (row_off[:, None] + col_off[None, :]).long()]        # (B, n, n), image orientation
+    r = (depth.double() - t.double()).view(B, -1, 1)
+    J = jac.double().view(B, -1, 12)
+    wJ = J if weight is None else J * weight.detach().double().reshape(B, -1, 1)
+    M = torch.bmm(wJ.transpose(1, 2), torch.cat([J, r], dim=2))                 # (B, 12, 13): [J^T W J | J^T W r]
+    wr = r if weight is None else r * weight.detach().double().reshape(B, -1, 1)
+    energy = (wr * r).sum(dim=(1, 2))
+    return energy, (2.0 * M[:, :, 12]).to(pred.dtype), M[:, :, :12].contiguous()
+
+
 def field(params: torch.Tensor, n: int, step: float, z0: float, mode: int, sharpness: float = 0.0) -> torch.Tensor:
     """Full (B, n, n, n) fp32 grid: mode 0 = F (ins_outs), mode 1 = occupancy sigmoid(sharpness (1 - F))."""
     _require_cuda(params, "params")

@@ -388,32 +388,14 @@ struct Bwd {
     float ge[2];      // W F H2,  W F eG H1
 };
 
-// Option SQ_MERGED_RCP: the five reciprocals (1 + t1, 1 + t2, sx, sy, sz) from ONE MUFU.RCP of their product plus 12 multiplications:
-// on B200 a MUFU warp instruction costs ~6 issue cycles and an FMUL ~0.9 (profiles/peaks_r01.json), and the kernels are
-// bound by instruction dispatch.  The product cannot leave fp32 range: 1 + t is in [1, 2], and of the three
-// coordinates of a gradient-carrying point (F ~ 1) at most two are small, each at least ~1e-15 when not exactly 0.
-// Measured: no gain for the implicit kernel, 2.5 % slower for the explicit one (longer dependent chain) -> off.
-template <bool FIX = true>
+// Five reciprocals from one MUFU.RCP of their product: measured no faster, explicit kernel 2.5 % slower (profiles/tune_r01.txt).
 SQ_HD void point_backward(const Fwd& f, float W, Bwd& b) {
     const float WF = W * f.F;
-    float sx = f.sx, sy = f.sy, sz = f.sz;
-    bool zx = false, zy = false, zz = false;
-    if (FIX) {          // exact zeros: the fix-up replaces s^2 by a constant, so no gradient reaches s or a through that term
-        zx = (sx == 0.0f); zy = (sy == 0.0f); zz = (sz == 0.0f);
-        sx = zx ? 1.0f : sx; sy = zy ? 1.0f : sy; sz = zz ? 1.0f : sz;
-    }
-#ifdef SQ_MERGED_RCP
-    const float p1 = 1.0f + f.t1, p2 = 1.0f + f.t2;
-    const float pa = p1 * p2, pb = sx * sy, pc = pb * sz;
-    const float inv = rcp(pa * pc);
-    const float ia = inv * pc, ic = inv * pa;              // 1 / (p1 p2), 1 / (sx sy sz)
-    const float r1 = ia * p2, r2 = ia * p1;
-    const float ib = ic * sz;                              // 1 / (sx sy)
-    const float isx = ib * sy, isy = ib * sx, isz = ic * pb;
-#else
+    // exact zeros: the fix-up replaces s^2 by a constant, so no gradient reaches s or a through that term
+    const bool zx = (f.sx == 0.0f), zy = (f.sy == 0.0f), zz = (f.sz == 0.0f);
+    const float sx = zx ? 1.0f : f.sx, sy = zy ? 1.0f : f.sy, sz = zz ? 1.0f : f.sz;
     const float r1 = rcp(1.0f + f.t1), r2 = rcp(1.0f + f.t2);
     const float isx = rcp(sx), isy = rcp(sy), isz = rcp(sz);
-#endif
     const float s1 = f.t1 * r1, s2 = f.t2 * r2;
     const bool a_big = f.d1 >= 0.0f, e_big = f.d2 >= 0.0f;
     const float aD = a_big ? r1 : s1, bD = a_big ? s1 : r1;
@@ -422,19 +404,12 @@ SQ_HD void point_backward(const Fwd& f, float W, Bwd& b) {
     const float wx = wxy * aD, wy = wxy * bD;
     b.ge[0] = WF * fmaf(s2, fabsf(f.d2), f.h2);
     b.ge[1] = wxy * fmaf(s1, fabsf(f.d1), f.h1);
-    if (FIX) {
-        b.wa[0] = zx ? 0.0f : wx;
-        b.wa[1] = zy ? 0.0f : wy;
-        b.wa[2] = zz ? 0.0f : wz;
-        b.gs[0] = zx ? 0.0f : wx * isx;
-        b.gs[1] = zy ? 0.0f : wy * isy;
-        b.gs[2] = zz ? 0.0f : wz * isz;
-    } else {            // the caller knows no coordinate of this column can be exactly 0 (column_zero_possible)
-        b.wa[0] = wx; b.wa[1] = wy; b.wa[2] = wz;
-        b.gs[0] = wx * isx;
-        b.gs[1] = wy * isy;
-        b.gs[2] = wz * isz;
-    }
+    b.wa[0] = zx ? 0.0f : wx;
+    b.wa[1] = zy ? 0.0f : wy;
+    b.wa[2] = zz ? 0.0f : wz;
+    b.gs[0] = zx ? 0.0f : wx * isx;
+    b.gs[1] = zy ? 0.0f : wy * isy;
+    b.gs[2] = zz ? 0.0f : wz * isz;
 }
 
 // a harmless point for lanes that carry no gradient but run the backward with their warp (weight 0)
@@ -536,16 +511,7 @@ SQ_HD double log2_acc(double m, const RefTabs& tb) {
 constexpr float kRefine = SQ_KREFINE;     // |x| below which a gradient-carrying point is re-evaluated in fp64
 
 // One point in fp64: s = base + cf d (d_i = Ms[i][2] step), the forward chain of point_forward() and x = kl (F - 1).
-#ifdef SQ_REFINE_NOINLINE
-#if defined(__CUDACC__)
-__host__ __device__ __noinline__
-#else
-inline
-#endif
-#else
-SQ_HD
-#endif
-float refined_x(const Sample& S, double step, float kl, double b0, double b1, double b2, float cf, const RefTabs& tb) {
+SQ_HD float refined_x(const Sample& S, double step, float kl, double b0, double b1, double b2, float cf, const RefTabs& tb) {
     const double c = f2d(cf);
     double s0 = fma(c, S.Ms[2] * step, b0), s1 = fma(c, S.Ms[5] * step, b1), s2 = fma(c, S.Ms[8] * step, b2);
     if (S.zpack) {                                            // planes of exact zeros (zero_planes()): cf is an exact integer there
@@ -672,9 +638,6 @@ constexpr float kExplicitVjpBits = 36.0f;
 // so F < bound^2 also confines the point to the ellipsoid  w (sx^2 + sy^2) + sz^2 < bound^2 2^(1-e1), whose
 // intersection with the column is the root interval of a quadratic in the plane index.  Box and ellipsoid together
 // leave 15 % fewer planes to walk on BASELINE config 2 (exact level-set ranges would leave 29 % fewer).
-#ifndef SQ_NO_QUADRIC
-#define SQ_QUADRIC 1
-#endif
 
 // inclusive z-index range [c_lo, c_hi] outside which F >= bound^2; empty when c_hi < c_lo
 SQ_HD void column_range(const Sample& S, const Grid& g, float bound, const float* bh, int& c_lo, int& c_hi) {
@@ -684,20 +647,15 @@ SQ_HD void column_range(const Sample& S, const Grid& g, float bound, const float
         lo = fmaxf(lo, fminf(u, v));       // fminf/fmaxf drop the NaN of 0 * inf
         hi = fminf(hi, fmaxf(u, v));
     }
-#ifdef SQ_QUADRIC
-    {
-        // alpha c^2 + 2 beta c + gamma < 0 with s(c) = bh + c dh; 0.4 % of slack on the radius^2 on top of the 0.2 % in
-        // `bound` covers the fp32 evaluation (|bh| <= ~30: relative 1e-6 on the discriminant)
-        const float qB = bound * bound * 1.004f * S.qB1;
-        const float beta = fmaf(S.wd[0], bh[0], fmaf(S.wd[1], bh[1], S.wd[2] * bh[2]));
-        const float gamma = fmaf(S.qw, fmaf(bh[0], bh[0], bh[1] * bh[1]), fmaf(bh[2], bh[2], -qB));
-        const float disc = fmaf(beta, beta, -S.qa * gamma);
-        const float sq = sqrt_approx(fmaxf(disc, 0.0f));
-        const float u = (-beta - sq) * S.qia, v = (sq - beta) * S.qia;
-        lo = fmaxf(lo, u);
-        hi = fminf(hi, disc > 0.0f ? v : -1e30f);           // no real roots: the column misses the ellipsoid
-    }
-#endif
+    // alpha c^2 + 2 beta c + gamma < 0 with s(c) = bh + c dh; 0.4 % of slack on the radius^2 on top of the 0.2 % in
+    // `bound` covers the fp32 evaluation (|bh| <= ~30: relative 1e-6 on the discriminant)
+    const float qB = bound * bound * 1.004f * S.qB1;
+    const float beta = fmaf(S.wd[0], bh[0], fmaf(S.wd[1], bh[1], S.wd[2] * bh[2]));
+    const float gamma = fmaf(S.qw, fmaf(bh[0], bh[0], bh[1] * bh[1]), fmaf(bh[2], bh[2], -qB));
+    const float disc = fmaf(beta, beta, -S.qa * gamma);
+    const float sq = sqrt_approx(fmaxf(disc, 0.0f));
+    lo = fmaxf(lo, (-beta - sq) * S.qia);
+    hi = fminf(hi, disc > 0.0f ? (sq - beta) * S.qia : -1e30f);     // no real roots: the column misses the ellipsoid
     // one plane of slack per side: rounding of the bounds, the lo parts of s, and plane 0 sitting at z0 not 0
     const float nf = (float)g.n;
     lo = fminf(fmaxf(lo - 1.0f, 0.0f), nf);
@@ -824,20 +782,6 @@ SQ_HD void warp_range(int n, int& c_lo, int& c_hi) {
     if (c_hi < c_lo) { c_lo = 0; c_hi = -1; }
 }
 
-// Can a scaled coordinate of this column be EXACTLY 0 on some plane?  s_i(c) = (bh_i + c dh_i) + (bl_i + c dl_i)
-// vanishes only where the hi part does to within the (2^-24 relative) lo part, i.e. at a plane index within ~1e-5 of
-// c* = -bh_i / dh_i.  Conservative (NaN/inf from dh_i = 0 count as "possible"); true for ~1e-3 of random columns.
-// Columns for which this is false skip the three "s == 0 -> |s| := 1e-2" selects per plane and the six in the backward.
-SQ_HD bool column_zero_possible(const Sample& S, const float* bh) {
-    bool m = false;
-    for (int i = 0; i < 3; ++i) {
-        const float cs = -bh[i] * S.idh[i];
-        const float r = cs - rintf(cs);
-        m = m || !(fabsf(r) > 1e-4f) || !(fabsf(cs - S.cf0) > 1e-4f);
-    }
-    return m;
-}
-
 // ---------------------------------------------------------------- ImplicitLoss: one column
 // classes.py:274-279.  Walk from the camera side (z index n-1) down to 0:
 //   o_c = sigmoid(k (1 - F_c)),  cs_c = running sum of o,  T_c = exp(-tau cs_c),  depth = 1 - sum_c T_c / n.
@@ -878,7 +822,7 @@ struct ColGrad {       // two-moment accumulators of one column
 // (tau/n) sum_c cs_c is carried along and used when the depth is tiny (relative error < 0.4% there).
 // [c_lo, c_hi]: the (warp-uniform) z range to walk, from column_range() / warp_range().
 // running state of one column walk
-// The warp's pool of gradient-carrying points (SQ_BWD_COMPACT), structure of arrays, `cap` slots shared by the warp's 32
+// The warp's pool of gradient-carrying points, structure of arrays, `cap` slots shared by the warp's 32
 // columns.  During the walk the lanes whose point carries gradient append to it together (two ballots per plane that has
 // any): points near the surface (|x| < kRefine, re-evaluated in fp64 later) fill the pool from the FRONT, the others from the
 // BACK, so after the walk the two lists are already compact -- entries [0, nr) and (top, cap - 1] -- and are dealt out to the
@@ -929,22 +873,19 @@ SQ_HD int entry_link(float tagged) { return (int)((f32_bits(tagged) >> 5) & 255u
 
 struct ColState {
     float csl, cssum, tsum, psh, seen, T;
-    // SQ_BWD_COMPACT: the warp's pool, front entries so far and the next free back slot (both warp-uniform), this column's
+    // the warp's pool, front entries so far and the next free back slot (both warp-uniform), this column's
     // latest front entry, whether a point of this column had to be handled on the spot because the pool was full
     BwdQueue q;
     int nr, top, head;
     bool spilled;
 };
 
-// SQ_BWD_COMPACT.  The backward block runs for the whole warp as soon as ONE lane carries gradient, and the surface
+// The compacted backward.  The backward block runs for the whole warp as soon as ONE lane carries gradient, and the surface
 // crosses the 32 columns of a patch on different planes: 5.7 of 32 lanes do on average (tools/timeline.py).  So during
 // the walk a gradient-carrying lane only notes (plane, prefix of T) in the warp's shared-memory pool; after the walk --
 // when the column's suffix weight U and the sign of (depth - target) are known -- the pooled points of all 32 columns
 // are dealt out evenly to the lanes, which redo the forward for their point and run the backward once, weighted,
 // straight into the item's sums.  Points that find the pool full fall back to the on-the-spot two-moment path.
-#if !defined(SQ_NO_BWD_COMPACT) && !defined(SQ_BWD_COMPACT)
-#define SQ_BWD_COMPACT 1
-#endif
 #ifndef SQ_BWD_DEPTH
 #define SQ_BWD_DEPTH 15       // pool slots per lane; 15 (not 16): five blocks' pools fit one SM's shared memory (sqloss.cu SQ_IMPB_MINB)
 #endif
@@ -955,24 +896,19 @@ constexpr int kBwdPool = kBwdDepth * 32;      // slots of a warp's pool
 // geometry + forward chain + occupancy of one plane (independent of the scan state: two planes can be in flight)
 struct Plane { Fwd f; float x, eo, o, cf; };
 
-template <bool FIX>
 SQ_HD void plane_forward(const Sample& S, const ImplicitParams& P, const float* bh, const float* bl, float cf, Plane& p) {
     p.cf = cf;
     float sx = fmaf(cf, S.dh[0], bh[0]) + fmaf(cf, S.dl[0], bl[0]);
     float sy = fmaf(cf, S.dh[1], bh[1]) + fmaf(cf, S.dl[1], bl[1]);
     float sz = fmaf(cf, S.dh[2], bh[2]) + fmaf(cf, S.dl[2], bl[2]);
-    point_forward<FIX>(S, sx, sy, sz, p.f);
+    point_forward<true>(S, sx, sy, sz, p.f);
     p.o = occupancy(p.f.F, P.kl, p.x, p.eo);
 }
 
-// SQ_F32X2: 0 = off, 1 = forward-only kernels (default), 2 = also the fwd+bwd kernel.  Measured (profiles/tune_r01.txt):
-// forward-only kernel -3.7 %; fwd+bwd kernel no gain (the register pairing costs as many moves as the packing saves).
-#ifndef SQ_F32X2
-#define SQ_F32X2 1
-#endif
-#if defined(__CUDA_ARCH__) && SQ_F32X2
+#if defined(__CUDA_ARCH__)
 // Packed fp32 (Blackwell fma/add/sub/mul.f32x2: two operations per issue slot).  The two planes in flight execute the same
 // sequence on different data, and the kernel is bound by issue slots, so their non-MUFU arithmetic is done pairwise.
+// Forward-only walk alone: measured 3.7 % faster there, no gain in the fwd+bwd kernel (profiles/tune_r01.txt).
 struct F2 { float x, y; };
 __device__ __forceinline__ F2 f2(float a, float b) { F2 r; r.x = a; r.y = b; return r; }
 #define SQ_F2_OP3(name, op) \
@@ -989,7 +925,6 @@ SQ_F2_OP2(sub2, "sub.rn.ftz.f32x2")
 SQ_F2_OP2(mul2, "mul.rn.ftz.f32x2")
 
 // plane_forward() for two planes at once
-template <bool FIX>
 __device__ __forceinline__ void plane_forward2(const Sample& S, const ImplicitParams& P, const float* bh, const float* bl,
                                                float cfa, float cfb, Plane& pa, Plane& pb) {
     pa.cf = cfa; pb.cf = cfb;
@@ -1001,10 +936,8 @@ __device__ __forceinline__ void plane_forward2(const Sample& S, const ImplicitPa
     pa.f.sx = s[0].x; pa.f.sy = s[1].x; pa.f.sz = s[2].x;
     pb.f.sx = s[0].y; pb.f.sy = s[1].y; pb.f.sz = s[2].y;
     F2 m[3] = {s[0], s[1], s[2]};
-    if (FIX) {
 #pragma unroll
-        for (int i = 0; i < 3; ++i) { m[i].x = (m[i].x == 0.0f) ? kAbsFix : m[i].x; m[i].y = (m[i].y == 0.0f) ? kAbsFix : m[i].y; }
-    }
+    for (int i = 0; i < 3; ++i) { m[i].x = (m[i].x == 0.0f) ? kAbsFix : m[i].x; m[i].y = (m[i].y == 0.0f) ? kAbsFix : m[i].y; }
     const F2 pxy = f2(S.pxy, S.pxy), one = f2(1.0f, 1.0f);
     const F2 lA = mul2(pxy, f2(lg2_abs(m[0].x), lg2_abs(m[0].y)));
     const F2 lB = mul2(pxy, f2(lg2_abs(m[1].x), lg2_abs(m[1].y)));
@@ -1032,7 +965,7 @@ __device__ __forceinline__ void plane_forward2(const Sample& S, const ImplicitPa
 #endif
 
 // scan step of one plane: transmittance, suffix-sum bookkeeping and (for gradient-carrying warps) the backward
-template <bool BWD, bool FIX, bool QUEUE>      // QUEUE: gradient-carrying points go to the lane's BwdQueue (SQ_BWD_COMPACT)
+template <bool BWD, bool QUEUE>      // QUEUE: gradient-carrying points go to the lane's BwdQueue
 SQ_HD void plane_scan(const ImplicitParams& P, const Plane& p, ColState& st, ColGrad& cg) {
 #if defined(__CUDA_ARCH__)
     SQ_COUNT_HOOK(0, 1);
@@ -1049,7 +982,6 @@ SQ_HD void plane_scan(const ImplicitParams& P, const Plane& p, ColState& st, Col
 #endif
             bool now = active;                  // lanes whose point is handled on the spot
             bool any_now = true;                // warp-uniform: does any lane have one
-#if defined(SQ_BWD_COMPACT)
             if (QUEUE) {
                 // all active lanes of this plane append together, in lane order: front slots for the points near the
                 // surface, back slots for the others
@@ -1090,9 +1022,7 @@ SQ_HD void plane_scan(const ImplicitParams& P, const Plane& p, ColState& st, Col
                     st.spilled = st.spilled || active;
                 }
             }
-            if (any_now)
-#endif
-            {
+            if (any_now) {
 #if defined(__CUDA_ARCH__)
                 SQ_COUNT_HOOK(1, 1);
 #endif
@@ -1101,7 +1031,7 @@ SQ_HD void plane_scan(const ImplicitParams& P, const Plane& p, ColState& st, Col
                 Fwd fa = p.f;
                 if (!now) fwd_neutral(fa);          // keep the other lanes finite
                 Bwd b;
-                point_backward<FIX>(fa, W, b);
+                point_backward(fa, W, b);
                 st.seen = now ? 1.0f : st.seen;
                 const float pp = st.psh;       // T in front of this point (since the first active one)
                 for (int i = 0; i < 3; ++i) {
@@ -1117,7 +1047,7 @@ SQ_HD void plane_scan(const ImplicitParams& P, const Plane& p, ColState& st, Col
     st.tsum += st.T;
 }
 
-// ---- the queued points after the walk (SQ_BWD_COMPACT), three steps; `at` = index of the entry in the queue arrays
+// ---- the queued points after the walk, three steps; `at` = index of the entry in the queue arrays
 // 1. refined entries: x from the fp64 chain, and the first-order change of the point's occupancy that goes with it
 SQ_HD void queue_store_refined(const BwdQueue& q, int at, float x0, float x1) {
     const float eo = ex2(x1), o = rcp(1.0f + eo), w = eo * o * o;
@@ -1165,16 +1095,18 @@ SQ_HD float queue_depth_shift(const BwdQueue& q, int head, float U) {
 // 32-column group that takes more gradient points than any workload of the parity fuzz has.)
 // 3. every entry: forward redone in fp32 for the ratios the backward needs (not amplified by k); weight o (1 - o) and
 // suffix weight from the queue.  sign = sign(depth - target) of the column.
+// (FIX, here and in implicit_column: the exact-zero fix-up is part of every walk; the host build's callers spell it out)
 template <bool FIX>
 SQ_HD void queue_entry_backward(const Sample& S, const float* bh, const float* bl, float cf,
                                 float w, float Sw, float sign, bool has, Bwd& b) {
+    static_assert(FIX, "the walks always apply the exact-zero fix-up");
     Fwd f;
     float sx = fmaf(cf, S.dh[0], bh[0]) + fmaf(cf, S.dl[0], bl[0]), sy = fmaf(cf, S.dh[1], bh[1]) + fmaf(cf, S.dl[1], bl[1]),
           sz = fmaf(cf, S.dh[2], bh[2]) + fmaf(cf, S.dl[2], bl[2]);
-    point_forward<FIX>(S, sx, sy, sz, f);
+    point_forward<true>(S, sx, sy, sz, f);
     float W = w * Sw * sign;
     if (!has) { fwd_neutral(f); W = 0.f; }
-    point_backward<FIX>(f, W, b);
+    point_backward(f, W, b);
 }
 
 // ILP: number of z planes whose (independent) forward chains are in flight per thread.  A column walk is a serial
@@ -1185,13 +1117,14 @@ SQ_HD void queue_entry_backward(const Sample& S, const float* bh, const float* b
 #endif
 
 template <bool BWD, bool FIX = true, bool QUEUE = false>
-// QUEUE (SQ_BWD_COMPACT): bwd_q / U_out / nr_io / top_io / spilled_out / head_out are used (see ColState; nr_io, top_io: the
+// QUEUE: bwd_q / U_out / nr_io / top_io / spilled_out / head_out are used (see ColState; nr_io, top_io: the
 // pool's front count and next free back slot, in and out -- the kernels start every column group at 0 and cap - 1, the host
 // build carries them from column to column of a group); colgrad11 then holds only what was handled on the spot.
 SQ_HD float implicit_column(const Sample& S, const Grid& g, const ImplicitParams& P,
                             const float* bh, const float* bl, int c_lo, int c_hi, int lane_lo, float* colgrad11,
                             const BwdQueue* bwd_q = nullptr, float* U_out = nullptr, int* nr_io = nullptr, int* top_io = nullptr,
                             bool* spilled_out = nullptr, int* head_out = nullptr) {
+    static_assert(FIX, "the walks always apply the exact-zero fix-up");
     // planes in front of the range: o = 0, cs = 0, T = 1 each
     ColState st;
     if (QUEUE) { st.q = *bwd_q; st.nr = *nr_io; st.top = *top_io; }
@@ -1217,9 +1150,9 @@ SQ_HD float implicit_column(const Sample& S, const Grid& g, const ImplicitParams
 #if SQ_IMP_ILP >= 2
     for (; !stop && c - (SQ_IMP_ILP - 1) >= c_lo; c -= SQ_IMP_ILP, cfi -= (float)SQ_IMP_ILP) {
         Plane p[SQ_IMP_ILP];
-#if defined(__CUDA_ARCH__) && SQ_F32X2 && SQ_IMP_ILP == 2
-        if (SQ_F32X2 >= 2 || !BWD) {
-            plane_forward2<FIX>(S, P, bh, bl, cfi, (c - 1 == 0) ? S.cf0 : cfi - 1.0f, p[0], p[1]);
+#if defined(__CUDA_ARCH__) && SQ_IMP_ILP == 2
+        if (!BWD) {
+            plane_forward2(S, P, bh, bl, cfi, (c - 1 == 0) ? S.cf0 : cfi - 1.0f, p[0], p[1]);
         } else
 #endif
         {
@@ -1227,24 +1160,20 @@ SQ_HD float implicit_column(const Sample& S, const Grid& g, const ImplicitParams
 #pragma unroll
 #endif
             for (int j = 0; j < SQ_IMP_ILP; ++j)
-                plane_forward<FIX>(S, P, bh, bl, (j > 0 && c - j == 0) ? S.cf0 : cfi - (float)j, p[j]);
+                plane_forward(S, P, bh, bl, (j > 0 && c - j == 0) ? S.cf0 : cfi - (float)j, p[j]);
         }
 #if defined(__CUDA_ARCH__)
 #pragma unroll
 #endif
-        for (int j = 0; j < SQ_IMP_ILP; ++j) plane_scan<BWD, FIX, QUEUE>(P, p[j], st, cg);
-#ifndef SQ_NO_EARLY_EXIT
+        for (int j = 0; j < SQ_IMP_ILP; ++j) plane_scan<BWD, QUEUE>(P, p[j], st, cg);
         stop = !SQ_ANY(st.csl > -kDeep && c - SQ_IMP_ILP >= lane_lo);
-#endif
     }
 #endif
     for (; !stop && c >= c_lo; --c, cfi -= 1.0f) {
         Plane p0;
-        plane_forward<FIX>(S, P, bh, bl, (c == 0) ? S.cf0 : cfi, p0);
-        plane_scan<BWD, FIX, QUEUE>(P, p0, st, cg);
-#ifndef SQ_NO_EARLY_EXIT
+        plane_forward(S, P, bh, bl, (c == 0) ? S.cf0 : cfi, p0);
+        plane_scan<BWD, QUEUE>(P, p0, st, cg);
         stop = !SQ_ANY(st.csl > -kDeep && c - 1 >= lane_lo);
-#endif
     }
     // planes behind the range (and planes left out by the early exit): o = 0, cs and T stay what they are
     const float nb = (float)(c + 1);
@@ -1300,53 +1229,6 @@ SQ_HD void acc_add_point(Acc& acc, const Bwd& b, float cf, float dx, float dy) {
 // range an SQ's occupancy is exactly 0 and its chain is not evaluated.
 struct Range { int lo, hi; };
 
-// SQ_EXP_PAIR: where both superquadrics are in range, their two forward chains -- the same instruction sequence on
-// different data and different per-sample constants -- run as packed fp32 pairs (true SQ in .x, predicted in .y).
-#ifndef SQ_EXP_PAIR
-#define SQ_EXP_PAIR 0
-#endif
-#if defined(__CUDA_ARCH__) && SQ_F32X2 && SQ_EXP_PAIR
-template <bool FIX>
-__device__ __forceinline__ void forward_pair(const Sample& Sa, const Sample& Sb, float kl, float cf,
-                                             const float* bha, const float* bla, const float* bhb, const float* blb,
-                                             Fwd& fa, Fwd& fb, float& oa, float& ob, float& xb, float& eb) {
-    const F2 c = f2(cf, cf);
-    F2 s[3];
-#pragma unroll
-    for (int i = 0; i < 3; ++i)
-        s[i] = add2(fma2(c, f2(Sa.dh[i], Sb.dh[i]), f2(bha[i], bhb[i])), fma2(c, f2(Sa.dl[i], Sb.dl[i]), f2(bla[i], blb[i])));
-    fa.sx = s[0].x; fa.sy = s[1].x; fa.sz = s[2].x;
-    fb.sx = s[0].y; fb.sy = s[1].y; fb.sz = s[2].y;
-    F2 m[3] = {s[0], s[1], s[2]};
-    if (FIX) {
-#pragma unroll
-        for (int i = 0; i < 3; ++i) { m[i].x = (m[i].x == 0.0f) ? kAbsFix : m[i].x; m[i].y = (m[i].y == 0.0f) ? kAbsFix : m[i].y; }
-    }
-    const F2 pxy = f2(Sa.pxy, Sb.pxy), one = f2(1.0f, 1.0f);
-    const F2 lA = mul2(pxy, f2(lg2_abs(m[0].x), lg2_abs(m[0].y)));
-    const F2 lB = mul2(pxy, f2(lg2_abs(m[1].x), lg2_abs(m[1].y)));
-    const F2 lC = mul2(f2(Sa.pz, Sb.pz), f2(lg2_abs(m[2].x), lg2_abs(m[2].y)));
-    const F2 d1 = sub2(lA, lB);
-    const F2 t1 = f2(ex2_neg_abs(d1.x), ex2_neg_abs(d1.y));
-    const F2 u1 = add2(t1, one);
-    const F2 h1 = f2(lg2(u1.x), lg2(u1.y));
-    const F2 lE = mul2(f2(Sa.e21, Sb.e21), add2(f2(fmaxf(lA.x, lB.x), fmaxf(lA.y, lB.y)), h1));
-    const F2 d2 = sub2(lE, lC);
-    const F2 t2 = f2(ex2_neg_abs(d2.x), ex2_neg_abs(d2.y));
-    const F2 u2 = add2(t2, one);
-    const F2 h2 = f2(lg2(u2.x), lg2(u2.y));
-    const F2 lG = add2(f2(fmaxf(lE.x, lC.x), fmaxf(lE.y, lC.y)), h2);
-    const F2 yy = mul2(f2(Sa.e1, Sb.e1), lG);
-    const F2 F = f2(ex2(yy.x), ex2(yy.y));
-    const F2 xx = fma2(F, f2(kl, kl), f2(-kl, -kl));
-    const F2 eo = f2(ex2(xx.x), ex2(xx.y));
-    const F2 v = add2(eo, one);
-    fa.d1 = d1.x; fa.t1 = t1.x; fa.h1 = h1.x; fa.d2 = d2.x; fa.t2 = t2.x; fa.h2 = h2.x; fa.lG = lG.x; fa.F = F.x;
-    fb.d1 = d1.y; fb.t1 = t1.y; fb.h1 = h1.y; fb.d2 = d2.y; fb.t2 = t2.y; fb.h2 = h2.y; fb.lG = lG.y; fb.F = F.y;
-    oa = rcp(v.x); ob = rcp(v.y); xb = xx.y; eb = eo.y;
-}
-#endif
-
 // one z plane of explicit_column; HAS_T / HAS_P: whether the true / predicted SQ can be occupied on this plane.
 // VJP (sq_occupancy_vjp): no true SQ, no squared difference; the point's weight is the upstream voxel `up` (dL/d o) and the
 // weight cut is `kact` bits (kExplicitVjpBits) instead of kActiveExplicit, and the z moment is taken about plane `zc`.
@@ -1360,12 +1242,6 @@ SQ_HD void explicit_step(const Sample& St, const Sample& Sp, float kl, float cf,
     static_assert(!VOX || VJP, "the voxel loss is a variant of the VJP walk");
     float ot = 0.f, op = 0.f, xp = 1e30f, ep = 0.f;
     Fwd ft, fp;
-#if defined(__CUDA_ARCH__) && SQ_F32X2 && SQ_EXP_PAIR
-    if (HAS_T && HAS_P) {
-        forward_pair<true>(St, Sp, kl, cf, bht, blt, bhp, blp, ft, fp, ot, op, xp, ep);
-    } else
-#endif
-    {
     if (HAS_T) {
         float sx = fmaf(cf, St.dh[0], bht[0]) + fmaf(cf, St.dl[0], blt[0]), sy = fmaf(cf, St.dh[1], bht[1]) + fmaf(cf, St.dl[1], blt[1]),
               sz = fmaf(cf, St.dh[2], bht[2]) + fmaf(cf, St.dl[2], blt[2]);
@@ -1378,7 +1254,6 @@ SQ_HD void explicit_step(const Sample& St, const Sample& Sp, float kl, float cf,
     }
     if (HAS_T) { float xt, et; ot = occupancy(ft.F, kl, xt, et); }
     if (HAS_P) op = occupancy(fp.F, kl, xp, ep);
-    }
     const float d = (VOX ? up : ot) - op;
     if (!VJP || VOX) sq = fmaf(d, d, sq);
     if (BWD && HAS_P) {

@@ -55,20 +55,10 @@ namespace {
 #ifndef SQ_IMPB_MINB
 // 5 blocks = 20 warps per SM at 96 registers (60 bytes of spill on cold paths): the phases of an item outside the z walk
 // are dependent chains (profiles/phases_r02.txt), and a fifth warp per scheduler hides more of them than the 26 registers
-// were worth -- 48.0 vs 49.2-50.1 us per call (profiles/tune_r02.txt run l).  It takes the three settings below with it:
-// the reduction tile aliased onto the queue arrays and a 15-deep queue (shared memory for 5 blocks), one deal-out chain
-// in flight instead of two (registers).  The round's earlier shape: -DSQ_IMPB_MINB=4 -DSQ_BWD_DEPTH=16 -DSQ_TILE_ALIAS=0
-// -DSQ_DENSE_ILP=2.
+// were worth -- 48.0 vs 49.2-50.1 us per call (profiles/tune_r02.txt run l).  Five blocks need the reduction tile
+// aliased onto the pool arrays and a 15-deep pool (shared memory), and one deal-out chain in flight instead of two
+// (registers); the round's earlier shape was -DSQ_IMPB_MINB=4 -DSQ_BWD_DEPTH=16.
 #define SQ_IMPB_MINB 5
-#endif
-#ifndef SQ_TILE_ALIAS
-#define SQ_TILE_ALIAS 1
-#endif
-#ifndef SQ_WALK_ESTIMATE     // cost classes of the implicit kernels from the planes a walk really visits (sq_core.cuh footprint_walk)
-#define SQ_WALK_ESTIMATE 1
-#endif
-#ifndef SQ_DENSE_ILP
-#define SQ_DENSE_ILP 1
 #endif
 #ifndef SQ_IMPB_CPT
 #define SQ_IMPB_CPT 1
@@ -261,21 +251,6 @@ size_t scratch_layout(int batch, int n, char* base, Scratch* s) {
         s->queue_cap = (int)cap;
     }
     return off;
-}
-
-// ------------------------------------------------------------------------------------------------ PDL
-// Programmatic dependent launch (-DSQ_PDL): the column kernel and the finalize kernel are launched with the
-// programmatic-stream-serialization attribute, so their blocks can become resident while the preceding kernel of the call
-// drains; pdl_wait() returns once that kernel has completed and its writes are visible.
-__device__ __forceinline__ void pdl_wait() {
-#ifdef SQ_PDL
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
-}
-__device__ __forceinline__ void pdl_trigger() {
-#ifdef SQ_PDL
-    asm volatile("griddepcontrol.launch_dependents;");
-#endif
 }
 
 // ------------------------------------------------------------------------------------------------ prep / plan
@@ -775,9 +750,6 @@ __device__ unsigned long long g_phase[8];
 #define SQ_PH(i) do { } while (0)
 #endif
 
-#ifndef SQ_EARLY_MARGIN      // measured (profiles/tune_r02.txt run k): margins 1..3 are 1-2 us SLOWER per call than none -> off
-#define SQ_EARLY_MARGIN 0
-#endif
 // dynamic shared memory of the fwd+bwd kernel, per warp: the pool's 4 float arrays + 11 x 32 column values
 constexpr size_t kImplicitBwdSmemPerWarp = (size_t)kBwdPool * 4 * sizeof(float) + 11 * 32 * sizeof(float);
 static_assert(kImplicitBwdSmemPerWarp % 32 == 0, "per-warp regions stay 32-byte aligned (BwdQueue::where carries the lane in its low bits)");
@@ -805,34 +777,22 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
     constexpr bool JAC = sizeof...(Jac) > 0;
     static_assert(!JAC || (BWD && !VJP && CPTMAX == 1), "the Jacobian mode is a mode of the fwd+bwd kernel");
     __shared__ Sample Ssh[THREADS / 32];
-#if SQ_TILE_ALIAS && defined(SQ_BWD_COMPACT)
     // the fwd+bwd kernel's reduction tile lives in the warp's pool arrays, which are dead by the time the item's sums
     // are put there (one column group per item only): shared memory for 5 blocks per SM
-    static_assert(!BWD || CPTMAX == 1, "SQ_TILE_ALIAS needs one column group per work item");
+    static_assert(!BWD || CPTMAX == 1, "the reduction tile in the pool needs one column group per work item");
     static_assert(4 * kBwdPool >= kRedFloats, "pool arrays too small to hold the tile");
     __shared__ __align__(16) float tiles_static[BWD ? 1 : THREADS / 32][kRedFloats];
-#else
-    __shared__ __align__(16) float tiles_static[THREADS / 32][kRedFloats];
-#endif
-#ifdef SQ_BWD_COMPACT       // per warp, in dynamic shared memory (BWD only; implicit_bwd_smem_bytes): the pool of gradient-carrying
-                            // points (BwdQueue arrays), per-column data for them
+    // per warp, in dynamic shared memory (BWD only; implicit_bwd_smem_bytes): the pool of gradient-carrying points (BwdQueue
+    // arrays), per-column data for them
     constexpr int kQN = kBwdPool;
     extern __shared__ __align__(32) unsigned char dyn_smem[];
     float* const qbuf = reinterpret_cast<float*>(dyn_smem + (size_t)(threadIdx.x >> 5) *
                                                  (kImplicitBwdSmemPerWarp + (JAC ? kJacStageBytesPerWarp : 0)));    // [4][kQN]
     float* const colinfo_w = qbuf + 4 * kQN;                                                                         // [11][32]
-#else
-    static_assert(!JAC, "the Jacobian mode needs SQ_BWD_COMPACT");
-#endif
-#if SQ_TILE_ALIAS && defined(SQ_BWD_COMPACT)
     float* const tile_w = BWD ? qbuf : tiles_static[threadIdx.x >> 5];
-#else
-    float* const tile_w = tiles_static[threadIdx.x >> 5];
-#endif
     static_assert(!VJP || BWD, "the VJP mode is a mode of the fwd+bwd kernel");
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     Sample& S = Ssh[warp];
-#if defined(SQ_BWD_COMPACT) && !defined(SQ_TABLES_GLOBAL)
     // the tables of the fp64 refinement, copied to shared memory once per block (3 KB; they are read with per-lane indices)
     __shared__ __align__(16) double tabs[BWD ? 384 : 130];      // (forward-only: never read)
     constexpr int kTabRegs = (384 + THREADS - 1) / THREADS;
@@ -845,16 +805,11 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
         }
     }
     const RefTabs tb{tabs, tabs + 128};
-#else
-    const RefTabs tb = default_tabs();
-#endif
     // Persistent warps pull work items from a global cursor, most expensive first (plan kernel).  The next item and its
     // Sample are fetched while the current item is processed.  No block-level barrier anywhere.
     // Items the plan kernel has proven empty are never touched: depth is exactly 0 on all their columns (depth_out was
     // cleared by the host), their loss sum |target| is part of the per-sample offset the plan kernel computed, their
     // partial rows were zeroed there.  What this kernel accumulates as "loss" is |depth - t| - |t| per walked column.
-    pdl_wait();                                           // the plan kernel's Samples, queues and counters
-    pdl_trigger();                                        // the finalize kernel may become resident (it waits for this grid)
 #ifdef SQ_TIMELINE
     const unsigned long long t_begin = gtime();
     unsigned long long t_last_fetch = t_begin, n_items = 0;
@@ -868,13 +823,11 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
     {
         SampleFetch pre;
         if (wp.item >= 0) pre.fetch(samples + L.sample_of(wp.item), lane);
-#if defined(SQ_BWD_COMPACT) && !defined(SQ_TABLES_GLOBAL)
         if (BWD) {
 #pragma unroll
             for (int r = 0; r < kTabRegs; ++r) { const int i = threadIdx.x + r * THREADS; if (i < 384) tabs[i] = tab_reg[r]; }
             __syncthreads();                               // the only block-level barrier: every warp passes here once
         }
-#endif
         while (wp.item >= 0) {
 #ifdef SQ_TIMELINE
             t_last_fetch = gtime(); ++n_items;
@@ -911,9 +864,6 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
             }
 #pragma unroll 1
             for (int k = 0; k < L.cpt; ++k) {
-#ifdef SQ_EARLY_CLAIM
-                if (k == L.cpt - 1 && wp.claim(lane)) pre.fetch(samples + L.sample_of(wp.next), lane);
-#endif
                 const int ia = it.ia, ib = it.ib;
                 const bool valid = it.valid(L);
                 const int row = g.n - 1 - ib, col = ia;        // classes.py:279: img[row, col] = depth[x = col, y = n-1-row]
@@ -928,9 +878,7 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
                 const int own_lo = c_hi >= c_lo ? c_lo : g.n;  // this lane's own range (the early exit of the walk looks at it)
                 warp_range(g.n, c_lo, c_hi);
                 if (c_hi < c_lo) {                             // warp-uniform: no occupancy anywhere, depth is exactly 0
-#ifndef SQ_EARLY_CLAIM
                     if (k == L.cpt - 1 && wp.claim(lane)) pre.fetch(samples + L.sample_of(wp.next), lane);
-#endif
                     continue;
                 }
                 SQ_COUNT_HOOK(5, 1);
@@ -938,57 +886,28 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
 #ifdef SQ_ITEMLOG
                 const long long il_w0 = clock64();
 #endif
-#if defined(SQ_BWD_COMPACT) && !defined(SQ_NO_STAGED_CLAIM) && !defined(SQ_EARLY_CLAIM) && SQ_EARLY_MARGIN > 0
-                // Far from the end of the queue the cursor atomic goes out BEFORE the walk (its L2 round trip then costs
-                // nothing); in the end-game -- fewer than SQ_EARLY_MARGIN items per warp left -- an item claimed before a
-                // long walk would be work no idle warp can take, so the claim waits until after the walk (see below).
-                const bool early = BWD && k == L.cpt - 1 &&
-                                   wp.item_pos + SQ_EARLY_MARGIN * (int)(gridDim.x * (THREADS / 32)) < wp.total;
-                if (early) wp.claim_issue(lane);
-#else
-                const bool early = false;
-#endif
                 float bh[3], bl[3], cg[11], dxy[2];
                 column_base(S, g, valid ? ia : 0, valid ? ib : 0, bh, bl, dxy);
-                float depth;
-#ifndef SQ_FIXHOIST      // hoisting the exact-zero fix-up out of the walk (two copies of the loop): measured 1 us
-                         // SLOWER per call once everything else was in place (profiles/tune_r01.txt) -> off
-#ifdef SQ_BWD_COMPACT
                 // (the entries' tags sit in the plane index's low mantissa bits: small integers, and plane 0's own "index" below 1)
                 const int pool = (g.n <= kPoolMaxPlanes && S.cf0 < 1.0f) ? kQN : 0;
                 float U = 0.f; int nr = 0, top = pool - 1, head = kNoLink; bool spilled = false;
                 unsigned where = (unsigned)__cvta_generic_to_shared(qbuf) | (unsigned)lane;
                 asm volatile("" : "+r"(where));                       // kept in a register (sq_core.cuh plane_scan)
                 const BwdQueue qwarp{qbuf, qbuf + kQN, qbuf + 2 * kQN, qbuf + 3 * kQN, pool, lane, where};
-                depth = implicit_column<BWD, true, BWD>(S, g, P, bh, bl, c_lo, c_hi, own_lo, cg, &qwarp, &U, &nr, &top, &spilled, &head);
-#else
-                depth = implicit_column<BWD, true>(S, g, P, bh, bl, c_lo, c_hi, own_lo, cg);
-#endif
-#else
-                if (__any_sync(0xffffffffu, column_zero_possible(S, bh)))
-                    depth = implicit_column<BWD, true>(S, g, P, bh, bl, c_lo, c_hi, own_lo, cg);
-                else
-                    depth = implicit_column<BWD, false>(S, g, P, bh, bl, c_lo, c_hi, own_lo, cg);
-#endif
+                // (exact-zero fix-up inside the walk: a second loop copy without it measured 1 us slower, profiles/tune_r01.txt)
+                const float depth = implicit_column<BWD, true, BWD>(S, g, P, bh, bl, c_lo, c_hi, own_lo, cg, &qwarp, &U, &nr, &top,
+                                                                    &spilled, &head);
                 SQ_PH(1);
 #ifdef SQ_ITEMLOG
                 il_walk += clock64() - il_w0;
 #endif
-#ifndef SQ_EARLY_CLAIM
                 // Claim the next item only now, after the walk: the cursor -> queue -> Sample chain then stalls this warp
                 // for ~1300 cycles, but the kernel is bound by instruction dispatch and the other warps of the scheduler
                 // fill the gap; an item claimed at the start of a long walk, on the other hand, is work no idle warp can
                 // take -- during the end-game that was the tail of the kernel.
-#if defined(SQ_BWD_COMPACT) && !defined(SQ_NO_STAGED_CLAIM)
                 const bool staged = BWD && k == L.cpt - 1;     // fwd+bwd: the claim is spread over the backward passes
-                if (staged) { if (!early) wp.claim_issue(lane); }
-                else
-#else
-                const bool staged = false;
-#endif
-                if (k == L.cpt - 1 && wp.claim(lane)) pre.fetch(samples + L.sample_of(wp.next), lane);
-#endif
-#if defined(SQ_BWD_COMPACT)
+                if (staged) wp.claim_issue(lane);
+                else if (k == L.cpt - 1 && wp.claim(lane)) pre.fetch(samples + L.sample_of(wp.next), lane);
                 if (BWD) {
                     // sign of (depth - target) per column (VJP: the upstream pixel); 0 for masked lanes
                     float wsg = 0.f;
@@ -1016,12 +935,10 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
 #ifdef SQ_ITEMLOG
                     il_q += total + (any_spill ? 1000 : 0); il_qr += total_r;
 #endif
-#ifndef SQ_EARLY_CLAIM
                     if (staged) {
                         wp.claim_lookup(lane);
                         if (total == 0 && wp.claim_finish()) pre.fetch(samples + L.sample_of(wp.next), lane);
                     }
-#endif
                     SQ_PH(2);
                     if (total > 0 || any_spill) {
                         Acc acc;
@@ -1050,15 +967,9 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
                             __syncwarp();
                             SQ_PH(3);
                             const float tau = P.tl * (float)kLn2;
-#ifdef SQ_DEPTH_SHIFT       // the refined occupancies' first-order effect on the rendered depth: measured below the loss's other
-                            // fp32 errors on every workload (profiles/tune_r02.txt) and 2 us per call -> off
-                            if (!VJP && head != kNoLink) loss_sum = fmaf(wsg * tau * g.inv_n, queue_depth_shift(qwarp, head, U), loss_sum);
-#endif
-#ifndef SQ_EARLY_CLAIM
                             if (staged && wp.claim_finish()) pre.fetch(samples + L.sample_of(wp.next), lane);
-#endif
                             // 2. + 3. all entries, dealt out evenly: suffix weight (corrected for the refined entries of the
-                            // entry's column), forward redone, backward; two rounds in flight (two independent MUFU chains)
+                            // entry's column), forward redone, backward
                             auto dealt = [&](int j, Bwd& bq, float& cfq, float& dx_, float& dy_) {
                                 const bool has = j < total;
                                 // front entries first, then the back ones from the pool's end; idle lane of the last round: a
@@ -1098,15 +1009,6 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
                                     __syncwarp();
                                 }
                             }
-#if SQ_DENSE_ILP == 2
-                            for (; j - lane + 32 < total; j += 64) {
-                                Bwd b0, b1; float c0, c1, x0, x1, y0, y1;
-                                dealt(j, b0, c0, x0, y0);
-                                dealt(j + 32, b1, c1, x1, y1);
-                                acc_add_point(acc, b0, c0, x0, y0);
-                                acc_add_point(acc, b1, c1, x1, y1);
-                            }
-#endif
                             for (; j - lane < total; j += 32) {
                                 Bwd b0; float c0, x0, y0;
                                 dealt(j, b0, c0, x0, y0);
@@ -1140,27 +1042,14 @@ implicit_kernel(const SampleFull* __restrict__ samples, Grid g, Layout L, Implic
                         }
                         SQ_PH(5);
                     }
-                } else
-#endif
-                if (valid) {
-                    if (depth_out && !VJP) depth_out[((size_t)b * g.n + row) * g.n + col] = depth;
+                } else if (valid) {
+                    if (depth_out) depth_out[((size_t)b * g.n + row) * g.n + col] = depth;
                     if (target) {
                         float tv = tvs[0];
 #pragma unroll
                         for (int q = 1; q < CPTMAX; ++q) tv = k == q ? tvs[q] : tv;
                         asm volatile("" : "+f"(tv));           // first touch of the pixel after the walk (see above)
-                        const float diff = VJP ? tv : depth - tv;
-                        if (!VJP) loss_sum += fabsf(diff) - fabsf(tv);
-                        if (BWD && diff != 0.f) {
-                            float v[kRedStride];
-                            Acc acc;
-                            if (folded) { tile_get(tile_w, v); array_to_acc(v, acc); } else acc_zero(acc);
-                            implicit_fold(acc, cg, VJP ? diff : (diff > 0.f ? 1.f : -1.f), dxy[0], dxy[1]);
-                            acc_to_array(acc, v);
-                            v[18] = v[19] = 0.f;
-                            tile_put(tile_w, v);
-                            folded = true;
-                        }
+                        loss_sum += fabsf(depth - tv) - fabsf(tv);
                     }
                 }
             }
@@ -1587,10 +1476,9 @@ finalize_kernel(const SampleFull* __restrict__ samples, Grid g, int batch, int i
     __shared__ SampleFull S;
     __shared__ double wpart[kFinThreads / 32][kAccN];
     __shared__ double acc[kAccN];
-    // the sample's record (written by the plan / prep kernel) into shared memory, while the partial rows are on their way
+    // the sample's record (written by the plan / prep kernel) into shared memory
     for (int w = t; w < kFullWords; w += kFinThreads)
         reinterpret_cast<uint32_t*>(&S)[w] = __ldg(reinterpret_cast<const uint32_t*>(samples + b) + w);
-    pdl_wait();                                           // the column kernel's partial rows
     {
         double s[kAccN];
 #pragma unroll
@@ -1763,18 +1651,6 @@ int check_scratch(int batch, int n, void* scratch, size_t bytes, Scratch* s) {
     return 0;
 }
 
-// kernel launch that may overlap the tail of the preceding kernel in the stream (the kernel must call pdl_wait())
-template <typename... KArgs, typename... Args>
-cudaError_t launch_dependent(void (*kernel)(KArgs...), int grid, int block, size_t dyn_smem, cudaStream_t st, bool pdl, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)block); cfg.dynamicSmemBytes = dyn_smem; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
 int device_sm_count() {
     static int sms[64] = {0};
     int dev = 0;
@@ -1926,50 +1802,35 @@ static int implicit_loss_impl(const void* pred, int pred_dtype, int batch, int n
     const ImplicitParams P{sharpness * kLog2e, tau * kLog2e, implicit_cull_bound(sharpness * kLog2e), implicit_active_bits(sharpness * kLog2e, n, batch)};
     if (depth_out)      // the column kernel writes the depth only where a column group can hold occupancy
         SQ_TRY(cudaMemsetAsync(depth_out, 0, sizeof(float) * (size_t)batch * n * n, st));
-#ifdef SQ_SKIP_COLUMN      // timing experiment: without the column kernel nobody restores the control block
-    SQ_TRY(cudaMemsetAsync(s.ctl, 0, sizeof(Control), st));
-#endif
     const PlanTarget pt{target, target_stride_b, row_off, col_off};
     rc = launch_plan(pred, nullptr, pred_dtype, batch, true, g, L, P.bound, s, nullptr, target ? s.item_class : nullptr,
-                     target ? &pt : nullptr, st, heads, SQ_WALK_ESTIMATE ? 32.0f / P.tl : 0.f);
+                     target ? &pt : nullptr, st, heads, 32.0f / P.tl);
     if (rc) return rc;
     const int items = batch * L.rows_per_sample;
     const int* queue = L.rows_per_sample <= kPlanMaxItems ? s.queue : nullptr;
-#ifdef SQ_PDL
-    const bool pdl = (t_ev_before == nullptr && t_ev_after == nullptr);   // an event record in between breaks the chain
-#else
-    const bool pdl = false;
-#endif
-#ifndef SQ_SKIP_COLUMN      // timing experiments only (tools/tune.py): leave out the column and / or finalize kernel
     {
         ColumnKernelTimer timer(st);
         if (grad_pred) {
             const int blocks = persistent_blocks(items, SQ_IMPB_THREADS / 32, SQ_IMPB_MINB);
             constexpr size_t dyn = kImplicitBwdSmemPerWarp * (SQ_IMPB_THREADS / 32);
             SQ_TRY((opt_in_dyn_smem<implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT>>(dyn)));
-            SQ_TRY(launch_dependent(implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT>, blocks, SQ_IMPB_THREADS, dyn, st, pdl,
-                                    s.pred, g, L, P, items, s.ctl, queue, s.queue_cap, target, target_stride_b, row_off, col_off,
-                                    s.partials, depth_out));
+            implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT><<<blocks, SQ_IMPB_THREADS, dyn, st>>>(
+                s.pred, g, L, P, items, s.ctl, queue, s.queue_cap, target, target_stride_b, row_off, col_off, s.partials, depth_out);
         } else {
             const int blocks = persistent_blocks(items, SQ_IMPF_THREADS / 32, SQ_IMPF_MINB);
-            SQ_TRY(launch_dependent(implicit_kernel<false, SQ_IMPF_THREADS, SQ_IMPF_MINB, SQ_IMPF_CPT>, blocks, SQ_IMPF_THREADS, 0, st, pdl,
-                                    s.pred, g, L, P, items, s.ctl, queue, s.queue_cap, target, target_stride_b, row_off, col_off,
-                                    s.partials, depth_out));
+            implicit_kernel<false, SQ_IMPF_THREADS, SQ_IMPF_MINB, SQ_IMPF_CPT><<<blocks, SQ_IMPF_THREADS, 0, st>>>(
+                s.pred, g, L, P, items, s.ctl, queue, s.queue_cap, target, target_stride_b, row_off, col_off, s.partials, depth_out);
         }
     }
     SQ_TRY(cudaGetLastError());
-#endif
-#ifndef SQ_SKIP_FINALIZE
     if (target) {
         const double nn = (double)n * n;
-        SQ_TRY(launch_dependent(finalize_kernel<FIN_IMPLICIT>, batch, kFinThreads, 0, st, pdl,
-                                s.pred, g, batch, L.rows_per_sample, s.partials, 1.0 / nn,
-                                -(double)sharpness * (double)tau / (nn * n * (double)batch), pred_dtype, grad_pred, s.per_sample,
-                                per_sample, loss_out, &s.ctl->ticket, s.tv_sum, queue ? s.item_class : nullptr,
-                                static_cast<double*>(nullptr)));
+        finalize_kernel<FIN_IMPLICIT><<<batch, kFinThreads, 0, st>>>(
+            s.pred, g, batch, L.rows_per_sample, s.partials, 1.0 / nn, -(double)sharpness * (double)tau / (nn * n * (double)batch),
+            pred_dtype, grad_pred, s.per_sample, per_sample, loss_out, &s.ctl->ticket, s.tv_sum, queue ? s.item_class : nullptr,
+            nullptr);
         SQ_TRY(cudaGetLastError());
     }
-#endif
     return 0;
 }
 
@@ -2005,32 +1866,23 @@ int sq_depth_projection_vjp(const void* pred, int pred_dtype, int batch, int n, 
     // the weight cut of one sample (batch 1): a VJP's gradient of sample b does not depend on the batch
     const ImplicitParams P{sharpness * kLog2e, tau * kLog2e, implicit_cull_bound(sharpness * kLog2e), implicit_active_bits(sharpness * kLog2e, n, 1)};
     rc = launch_plan(pred, nullptr, pred_dtype, batch, true, g, L, P.bound, s, nullptr, s.item_class, nullptr, st, false,
-                     SQ_WALK_ESTIMATE ? 32.0f / P.tl : 0.f);
+                     32.0f / P.tl);
     if (rc) return rc;
     const int items = batch * L.rows_per_sample;
     const int* queue = L.rows_per_sample <= kPlanMaxItems ? s.queue : nullptr;
-#ifdef SQ_PDL
-    const bool pdl = (t_ev_before == nullptr && t_ev_after == nullptr);
-#else
-    const bool pdl = false;
-#endif
     {
         ColumnKernelTimer timer(st);
         const int blocks = persistent_blocks(items, SQ_IMPB_THREADS / 32, SQ_IMPB_MINB);
         constexpr size_t dyn = kImplicitBwdSmemPerWarp * (SQ_IMPB_THREADS / 32);
         SQ_TRY((opt_in_dyn_smem<implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT, true>>(dyn)));
-        SQ_TRY(launch_dependent(implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT, true>, blocks, SQ_IMPB_THREADS, dyn,
-                                st, pdl, s.pred, g, L, P, items, s.ctl, queue, s.queue_cap, grad_depth, 0LL,
-                                static_cast<const int*>(nullptr), static_cast<const int*>(nullptr), s.partials,
-                                static_cast<float*>(nullptr)));
+        implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT, true><<<blocks, SQ_IMPB_THREADS, dyn, st>>>(
+            s.pred, g, L, P, items, s.ctl, queue, s.queue_cap, grad_depth, 0LL, nullptr, nullptr, s.partials, nullptr);
     }
     SQ_TRY(cudaGetLastError());
     // d depth / d o_c = (tau / n) S_c and d o / d F = -k o (1 - o): the column sums carry o (1 - o) S_c x upstream
-    SQ_TRY(launch_dependent(finalize_kernel<FIN_IMPLICIT>, batch, kFinThreads, 0, st, pdl,
-                            s.pred, g, batch, L.rows_per_sample, s.partials, 0.0, -(double)sharpness * (double)tau / (double)n,
-                            pred_dtype, grad_pred, s.per_sample, static_cast<double*>(nullptr), static_cast<double*>(nullptr),
-                            &s.ctl->ticket, static_cast<const double*>(nullptr), queue ? s.item_class : nullptr,
-                            static_cast<double*>(nullptr)));
+    finalize_kernel<FIN_IMPLICIT><<<batch, kFinThreads, 0, st>>>(
+        s.pred, g, batch, L.rows_per_sample, s.partials, 0.0, -(double)sharpness * (double)tau / (double)n, pred_dtype, grad_pred,
+        s.per_sample, nullptr, nullptr, &s.ctl->ticket, nullptr, queue ? s.item_class : nullptr, nullptr);
     SQ_TRY(cudaGetLastError());
     return 0;
 }
@@ -2053,25 +1905,18 @@ int sq_depth_projection_jacobian(const void* pred, int pred_dtype, int batch, in
     SQ_TRY(cudaMemsetAsync(jac, 0, sizeof(float) * 12 * (size_t)batch * n * n, st));
     if (depth_out) SQ_TRY(cudaMemsetAsync(depth_out, 0, sizeof(float) * (size_t)batch * n * n, st));
     rc = launch_plan(pred, nullptr, pred_dtype, batch, true, g, L, P.bound, s, nullptr, s.item_class, nullptr, st, false,
-                     SQ_WALK_ESTIMATE ? 32.0f / P.tl : 0.f);
+                     32.0f / P.tl);
     if (rc) return rc;
     const int items = batch * L.rows_per_sample;
     const int* queue = L.rows_per_sample <= kPlanMaxItems ? s.queue : nullptr;
-#ifdef SQ_PDL
-    const bool pdl = (t_ev_before == nullptr && t_ev_after == nullptr);
-#else
-    const bool pdl = false;
-#endif
     {
         ColumnKernelTimer timer(st);
         const int blocks = persistent_blocks(items, SQ_IMPB_THREADS / 32, SQ_IMPB_MINB);
         constexpr size_t dyn = (kImplicitBwdSmemPerWarp + kJacStageBytesPerWarp) * (SQ_IMPB_THREADS / 32);
         constexpr auto kernel = implicit_kernel<true, SQ_IMPB_THREADS, SQ_IMPB_MINB, SQ_IMPB_CPT, false, JacOut>;
         SQ_TRY((opt_in_dyn_smem<kernel>(dyn)));
-        SQ_TRY(launch_dependent(kernel, blocks, SQ_IMPB_THREADS, dyn, st, pdl, s.pred, g, L, P, items, s.ctl, queue,
-                                s.queue_cap, static_cast<const float*>(nullptr), 0LL, static_cast<const int*>(nullptr),
-                                static_cast<const int*>(nullptr), static_cast<float*>(nullptr), depth_out,
-                                JacOut{jac, -(double)sharpness * (double)tau / (double)n}));
+        kernel<<<blocks, SQ_IMPB_THREADS, dyn, st>>>(s.pred, g, L, P, items, s.ctl, queue, s.queue_cap, nullptr, 0LL, nullptr,
+                                                     nullptr, nullptr, depth_out, JacOut{jac, -(double)sharpness * (double)tau / (double)n});
     }
     SQ_TRY(cudaGetLastError());
     return 0;

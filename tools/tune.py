@@ -1,6 +1,6 @@
 """Build variants of libsqloss.so with different -D tunables on the GPU box and time the column kernels.
 
-    python tools/tune.py "SQ_IMP_MINB=2" "SQ_IMP_MINB=3" "SQ_IMP_MINB=3,SQ_MAX_CPT=4" ...
+    python tools/tune.py "" "SQ_IMPB_MINB=4" "SQ_IMPB_MINB=4,SQ_BWD_DEPTH=16" ...
 
 Each variant is compiled to /tmp and loaded with ctypes next to torch (no package import, so several variants can
 coexist in one process).  Prints one line per variant: kernel-only ms (sq_profile_events) for the implicit fwd+bwd,
